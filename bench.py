@@ -3,7 +3,7 @@
 (1600x1184, 1 reference + 4 source views, ndepths 48,8,8, 3 GRU iterations per stage) with the
 cost-volume hot path on hand-written sm_100a kernels.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision f32|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision f32|bf16] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one depth map (one pass of the whole cascade over
 one 5-view batch of synthetic images).  `value` = depth maps/s with the inputs resident in HBM;
@@ -42,7 +42,8 @@ LABELS = {"dtu": (METRIC, WORKLOAD),
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps; impl reference runs at most this many, stopping at --cpu-budget-s (the line reports the number run)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default=os.environ.get("EFFIMVS_PRECISION", "bf16x3"), choices=["f32", "bf16", "bf16x3"])
@@ -54,7 +55,29 @@ def parse():
     ap.add_argument("--profile-one", action="store_true",
                     help="3 warm eager forwards, then ONE forward between cudaProfilerStart/Stop and exit (for ncu --profile-from-start off)")
     ap.add_argument("--cpu-budget-s", type=float, default=240.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy: "
+                         "depth00 .. depth12 and photometric_confidence, float32, every pixel (about 20 MB at the DTU shape)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+def output_arrays(out):
+    """name -> copy of each output of one forward, taken where the tensors live (on the device: no host copy yet)"""
+    arrays = {"depth{:02d}".format(i): d.detach().clone() for i, d in enumerate(out["depth"])}
+    arrays["photometric_confidence"] = out["photometric_confidence"].detach().clone()
+    return arrays
+
+
+def dump_outputs(out_dir, arrays):
+    """output_arrays() as DIR/<name>.npy; the inputs are seeded, so two builds can be compared file by file"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy() if t.dtype == torch.float64 else t.float().numpy())
 
 
 def build_model(hotpath, device, ndepths):
@@ -190,10 +213,11 @@ def run_reference(a, rank, world):
     t_begin = time.perf_counter()
     done_w = 0
     last = 0.0
+    result = [None]
 
     def one():
         t0 = time.perf_counter()
-        model(s["imgs"], s["proj_matrices"], s["depth_values"])
+        result[0] = model(s["imgs"], s["proj_matrices"], s["depth_values"])
         return time.perf_counter() - t0
 
     with torch.no_grad():
@@ -207,6 +231,8 @@ def run_reference(a, rank, world):
                 break
             last = one()
             times.append(last)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, output_arrays(result[0]))
     done_k = len(times)
     total = sum(times)
     value = done_k / total
@@ -545,12 +571,15 @@ def run_ours(a, rank, world, local_rank):
                 graph = None
                 torch.cuda.synchronize()
 
+        last = [out]      # what the latest step returned: the graph's output tensors, or a new eager result per step
+
         def step():
             flush.zero_()
             if graph is not None:
                 graph.replay()
                 return out
-            return forward()
+            last[0] = forward()
+            return last[0]
 
         def barrier():
             if world > 1:
@@ -574,6 +603,8 @@ def run_ours(a, rank, world, local_rank):
 
         with ClockSampler(local_rank) as clk:
             ms_dev = timed(step, a.steps, max(a.warmup, 3))
+            # a device-side copy: the host copy and the file writes wait until the clocks are no longer sampled
+            dumped = output_arrays(last[0]) if a.dump_outputs and rank == 0 else None
 
             # end to end through the public API (effimvs_b200.pipeline.DepthMapPipeline): every step copies the
             # sample from pinned host memory to the device and reads depth + confidence back to the host; the
@@ -606,6 +637,9 @@ def run_ours(a, rank, world, local_rank):
             ms_e2e, d2h = e2e_timed(pin_u8)               # headline: 8-bit images over PCIe
             ms_e2e_f32, _ = e2e_timed(pin)                # the same with fp32 host images (4x the image bytes)
         h2d, h2d_f32 = pipe.h2d_bytes(pin_u8), pipe.h2d_bytes(pin)
+        if dumped is not None:
+            dump_outputs(a.dump_outputs, dumped)
+            del dumped
 
         # The same forward with fp32 products in every 2-D convolution (torch.backends.cudnn.allow_tf32 = False: cuDNN's fp32
         # kernels for the FPN and the update block, whose tensor-core kernel follows the same switch) -- the setting of the

@@ -59,6 +59,16 @@ def load_dtu_weights(m):
     assert not res.unexpected_keys and all("num_batches" in k for k in res.missing_keys), res
 
 
+def headline_sample(depths, conf, k=1024):
+    """A fixed sample of k pixels of each of the 13 depth maps and of the confidence map (flat indices i * 2654435761 mod n,
+    distinct for k <= n since the multiplier is prime) -> 14 float32 arrays; what tests/golden/headline_port.npz stores."""
+    out = []
+    for t in list(depths) + [conf]:
+        flat = t.detach().reshape(-1).float().cpu().numpy()
+        out.append(flat[(np.arange(k, dtype=np.int64) * 2654435761) % flat.size])
+    return out
+
+
 def rel_max(a, b):
     """max|a-b| / max|b|  -- the north_star's cost-volume metric (SURVEY.md section 7 'hard parts')."""
     return float((a - b).abs().max() / b.abs().max().clamp(min=1e-30))
