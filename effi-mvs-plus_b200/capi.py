@@ -75,6 +75,11 @@ SIGNATURES = {
     "effimvs_conv2d_tf32_supported": (_i, [_i, _i]),
     "effimvs_conv2d_tf32_packed_bytes": (_sz, [_i, _i]),
     "effimvs_conv2d_tf32_pack": (_i, [_p, _i, _i, _p, _p]),
+    "effimvs_conv2d_bf16x3_supported": (_i, [_i, _i]),
+    "effimvs_conv2d_bf16x3_packed_bytes": (_sz, [_i, _i]),
+    "effimvs_conv2d_bf16x3_pack": (_i, [_p, _i, _i, _p, _p]),
+    "effimvs_conv2d_bf16x3": (_i, [_p, C.c_longlong, _i, _p, C.c_longlong, _i, _p, _p, _i, _i, _i, _i, _i,
+                                   _p, C.c_longlong, _p, C.c_longlong, _p, C.c_longlong, _p]),
     "effimvs_conv2d_tf32": (_i, [_p, C.c_longlong, _i, _p, C.c_longlong, _i, _p, _p, _i, _i, _i, _i, _i,
                                  _p, C.c_longlong, _p, C.c_longlong, _p, C.c_longlong, _p]),
     "effimvs_gru_init_f32": (_i, [_p, C.c_longlong, _i, _i, _p, _p]),

@@ -14,7 +14,15 @@
 // tensor pipe ~130-170 clk of A-operand streaming whatever its N, so halving their number is what counts).  Activations are
 // rounded to nearest when staged (cvt.rn.satfinite: |x| > 65504 saturates -- the inputs of these layers are tanh / sigmoid
 // / relu outputs of O(1) -- and |x| < 6e-5 goes gradually to an absolute error of 3e-8), weights when packed.  Callers
-// that need fp32 products keep cuDNN.
+// that need fp32 products use the bf16x3 instantiations below or keep cuDNN.
+//
+// Precision bf16x3 (effimvs_conv2d_bf16x3*, opt-in): the arithmetic class of the 3-D nets' default mode (conv3d_tc.cu).
+// Every operand is carried as a pair hi = bf16_rn(x), lo = bf16_rn(x - hi) (x - hi is exact in fp32; together ~2^-16
+// relative), and each K step issues hi.hi + hi.lo + lo.hi into the same fp32 accumulator -- fp32's exponent range, no
+// saturation.  A staged input row holds the hi copy followed by the lo copy (each in the layout below), the packed
+// weights the hi image followed by the lo image (36 Cin Cout bytes, both resident); K phases are at most 32 channels so
+// that 64 -> 64 (147 KB of weights) fits one CTA per SM with three stages.  Operand precision is a template parameter:
+// the f16 instantiations compile to the same instructions as without it.
 //
 // Formulation ("row sweep", input stationary).  A unit is a strip of 128 output pixels x R consecutive output rows of
 // one image.  Input row i of the strip (130 pixels with the x halo, zero beyond the image) is staged ONCE in shared
@@ -36,6 +44,7 @@
 //                          ADD_RELU            out = relu(acc + addend[pixel])                (encoder tail: context term)
 //                          GRU_GATES           z = sigmoid(acc[:h] + b) -> zbuf;  out = sigmoid(acc[h:] + b) * h_prev
 //                          GRU_UPDATE          out = (1 - z) * out + z * tanh(acc + b)        (in place on the hidden state)
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 #include <algorithm>
@@ -59,6 +68,7 @@ constexpr int C2_THREADS = (C2_PROD_WARP0 + C2_PROD_WARPS) * 32;   // 416
 constexpr int C2_EPI_STRIDE = 144;                // bytes per pixel row of an epilogue warp's transpose buffer (32 channels + 16 pad)
 constexpr int C2_EPI_BYTES = 4 * 32 * C2_EPI_STRIDE;
 constexpr int C2_MAX_COUT = 128;
+constexpr int C2_F16 = 0, C2_BF16X3 = 1;          // operand precision (template parameter of the kernel)
 
 struct C2Params {
     const float* in0; long long ps0; int c0;     // channel segment 0: pointer to (pixel 0, channel 0), pixel stride in floats
@@ -154,6 +164,21 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t da, uint64_t
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
         ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accum) : "memory");
 }
+// bf16x3: three MMAs into one accumulator -- hi.hi, hi.lo (B's lo image blo16 units on), lo.hi (A's lo copy alo16 units
+// on); f16: the one MMA.  A and B are descriptors, the offsets in 16-byte units.
+template <int PREC>
+__device__ __forceinline__ void umma_op(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accum, uint32_t alo16, uint32_t blo16) {
+    umma_tf32(tmem_d, da, db, idesc, accum);
+    if (PREC == C2_BF16X3) {
+        umma_tf32(tmem_d, da, db + blo16, idesc, 1u);
+        umma_tf32(tmem_d, da + alo16, db, idesc, 1u);
+    }
+}
+// instruction descriptor per precision: bf16x3 sets A and B format to bf16 (bits 7-9, 10-12 = 1)
+template <int PREC>
+__device__ __forceinline__ uint32_t umma_idesc_p(int n) {
+    return umma_idesc_tf32(n) | (PREC == C2_BF16X3 ? (1u << 7) | (1u << 10) : 0u);
+}
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
@@ -203,6 +228,14 @@ __device__ __forceinline__ uint32_t pack_half2(unsigned long long pair) {
     uint32_t r;
     asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
     return r;
+}
+// two floats (low word first) -> packed bf16 hi = bf16_rn(x) and lo = bf16_rn(x - hi); no saturation (fp32's exponent range)
+__device__ __forceinline__ void split_bf16x2(unsigned long long pair, uint32_t& hi, uint32_t& lo) {
+    float a, b;
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(a), "=f"(b) : "l"(pair));
+    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(b), "f"(a));
+    const float ra = a - __uint_as_float(hi << 16), rb = b - __uint_as_float(hi & 0xffff0000u);
+    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(rb), "f"(ra));
 }
 __device__ __forceinline__ float to_tf32(float x) {
     uint32_t r;
@@ -340,10 +373,10 @@ __device__ __forceinline__ Unit unit_of(const C2Params& P, int u) {
     return t;
 }
 
-// One instantiation per (epilogue mode, channel groups of a K phase): every role of the kernel is a single-warp chain whose speed
+// One instantiation per (epilogue mode, channel groups of a K phase, operand precision): every role of the kernel is a single-warp chain whose speed
 // is its instruction count, and three CTAs x three roles share the SM's instruction cache -- a run-time mode switch, a generic item
 // mapping and the profiling switches of the first version cost measurably (see DESIGN, appendix A), so they are compile-time here.
-template <int MODE, int GROUPS>
+template <int MODE, int GROUPS, int PREC>
 __global__ void __launch_bounds__(C2_THREADS, 2)
 conv2d_tc_kernel(const __grid_constant__ C2Params P, const uint8_t* __restrict__ wpk) {
 #ifdef EFFIMVS_CONV2D_PROFILING
@@ -401,6 +434,7 @@ conv2d_tc_kernel(const __grid_constant__ C2Params P, const uint8_t* __restrict__
         const int px_per_item = groups >= 4 ? 8 : 16, px_items = (C2_ROWPX + px_per_item - 1) / px_per_item;
         const int n_items = px_items * (groups >= 4 ? groups >> 2 : 1);
         const int ps0i = (int)P.ps0, ps1i = (int)P.ps1;                  // a row of a map is < 2^31 floats
+        constexpr int NIT = PREC == C2_BF16X3 ? 4 : 5;                    // items in flight per lane (bf16x3: two stores each)
         uint32_t fill = 0;
         for (int u = blockIdx.x; u < P.n_units; u += gridDim.x) {
             const Unit t = unit_of(P, u);
@@ -417,11 +451,11 @@ conv2d_tc_kernel(const __grid_constant__ C2Params P, const uint8_t* __restrict__
                     const float* r0 = P.in0 + rowpix * P.ps0;          // (pixel 0 of the row, channel 0) of the two segments
                     const float* r1 = P.in1 + rowpix * P.ps1 - P.c0;
                     const int ch0 = p * KC + cgl0 * 8, xb = t.x0 - 1 + pxl;
-                    for (int it0 = pwg; it0 < n_items; it0 += 5 * P.gw) {
-                        F8 v[5];
-                        uint32_t off[5];
+                    for (int it0 = pwg; it0 < n_items; it0 += NIT * P.gw) {
+                        F8 v[NIT];
+                        uint32_t off[NIT];
 #pragma unroll
-                        for (int k = 0; k < 5; ++k) {
+                        for (int k = 0; k < NIT; ++k) {
                             const int it = it0 + P.gw * k;
                             v[k].a = v[k].b = v[k].c = v[k].d = 0ull;
                             off[k] = 0xffffffffu;
@@ -436,10 +470,17 @@ conv2d_tc_kernel(const __grid_constant__ C2Params P, const uint8_t* __restrict__
                             }
                         }
 #pragma unroll
-                        for (int k = 0; k < 5; ++k) {
+                        for (int k = 0; k < NIT; ++k) {
                             if (off[k] != 0xffffffffu) {
                                 uint4 q;
-                                q.x = pack_half2(v[k].a); q.y = pack_half2(v[k].b); q.z = pack_half2(v[k].c); q.w = pack_half2(v[k].d);
+                                if (PREC == C2_BF16X3) {
+                                    uint4 l;    // the lo copy sits GROUPS channel groups after the hi copy
+                                    split_bf16x2(v[k].a, q.x, l.x); split_bf16x2(v[k].b, q.y, l.y);
+                                    split_bf16x2(v[k].c, q.z, l.z); split_bf16x2(v[k].d, q.w, l.w);
+                                    *reinterpret_cast<uint4*>(dst + off[k] + GROUPS * C2_CG_BYTES) = l;
+                                } else {
+                                    q.x = pack_half2(v[k].a); q.y = pack_half2(v[k].b); q.z = pack_half2(v[k].c); q.w = pack_half2(v[k].d);
+                                }
                                 *reinterpret_cast<uint4*>(dst + off[k]) = q;
                             }
                         }
@@ -472,6 +513,8 @@ conv2d_tc_kernel(const __grid_constant__ C2Params P, const uint8_t* __restrict__
             const bool two_max = 3 * P.coutp > 256;                   // an MMA spans at most two of the three stacked row blocks
             const bool mma_on = !(dbg & 1);
             const uint32_t rm = (uint32_t)P.ring - 1u, rs = (uint32_t)__ffs(P.ring) - 1u;
+            constexpr uint32_t alo16 = (GROUPS * C2_CG_BYTES) >> 4;                 // bf16x3: lo copy of a staged row
+            const uint32_t blo16 = PREC == C2_BF16X3 ? (uint32_t)P.w_bytes >> 5 : 0u;  // bf16x3: lo weight image (second half)
             mbar_wait_warp(&bar_w, 0);
             __syncwarp();
             uint32_t fill = 0, seq_base = 0;
@@ -501,7 +544,7 @@ conv2d_tc_kernel(const __grid_constant__ C2Params P, const uint8_t* __restrict__
                     const int lenB = nt - lenA;
                     const uint32_t dA = tmem + (seq0 & rm) * coutp, dB = tmem + ((seq0 + (uint32_t)lenA) & rm) * coutp;
                     const uint32_t boffA = kyb0 * coutp, boffB = (kyb0 + (uint32_t)lenA) * coutp;          // 16-byte units (one per row)
-                    const uint32_t idA = umma_idesc_tf32(lenA * P.coutp), idB = umma_idesc_tf32(lenB * P.coutp), id1 = umma_idesc_tf32(P.coutp);
+                    const uint32_t idA = umma_idesc_p<PREC>(lenA * P.coutp), idB = umma_idesc_p<PREC>(lenB * P.coutp), id1 = umma_idesc_p<PREC>(P.coutp);
                     for (int p = 0; p < P.n_phases; ++p, ++fill) {
                         const uint32_t s = fill % S, n = fill / S;
                         mbar_wait_warp(&bar_afull[s], n & 1);
@@ -516,7 +559,7 @@ conv2d_tc_kernel(const __grid_constant__ C2Params P, const uint8_t* __restrict__
 #pragma unroll
                                 for (int k = 0; k < 3; ++k)
                                     if (k < nt)
-                                        umma_tf32(tmem + ((seq0 + k) & rm) * coutp, adesc0, bstep + (uint64_t)((kyb0 + k) * coutp), id1, ((fresh >> k) & 1u) ^ 1u);
+                                        umma_op<PREC>(tmem + ((seq0 + k) & rm) * coutp, adesc0, bstep + (uint64_t)((kyb0 + k) * coutp), id1, ((fresh >> k) & 1u) ^ 1u, alo16, blo16);
                                 q0 = 1;
                                 bstep += blk16;
                             }
@@ -526,8 +569,8 @@ conv2d_tc_kernel(const __grid_constant__ C2Params P, const uint8_t* __restrict__
                             for (int q = q0; q < 3 * ksteps; ++q, boff += blk16) {
                                 const int j = q / 3, kx = q - 3 * j;
                                 const uint64_t adesc = adesc0 + (uint64_t)(uint32_t)(j * 2 * (C2_CG_BYTES >> 4) + kx);
-                                umma_tf32(dA, adesc, bA + boff, idA, 1u);
-                                if (lenB > 0) umma_tf32(dB, adesc, bB + boff, idB, 1u);
+                                umma_op<PREC>(dA, adesc, bA + boff, idA, 1u, alo16, blo16);
+                                if (lenB > 0) umma_op<PREC>(dB, adesc, bB + boff, idB, 1u, alo16, blo16);
                             }
                         }
                         if (leader) {
@@ -643,72 +686,93 @@ __global__ void conv2d_pack_kernel(const float* __restrict__ w, int cin, int cou
         dst[i] = __float2half_rn(fminf(fmaxf(v, -65504.0f), 65504.0f));
     }
 }
-
-int pow2_cols(int n) { int c = 32; while (c < n) c <<= 1; return c; }
-// channels per K phase: the whole input when it is 16, 32 or 64 channels, else 32- or 16-channel phases
-int phase_channels(int cin) { return (cin == 16 || cin == 32 || cin == 64) ? cin : (cin % 32 == 0 ? 32 : 16); }
-
-}  // namespace
-}  // namespace effimvs
-
-using namespace effimvs;
-
-static long long* g_conv2d_timeline = nullptr;
-/* profiling hook (not part of include/effimvs.h): device buffer of 3 * 64 * 4 int64 that CTA 0 of the following launches fills */
-extern "C" void effimvs_conv2d_debug_timeline(void* buf) { g_conv2d_timeline = (long long*)buf; }
-
-extern "C" size_t effimvs_conv2d_tf32_packed_bytes(int cin, int cout) {
-    if (cin <= 0 || cout <= 0) return 0;
-    const int coutp = (cout + 15) / 16 * 16;
-    return (size_t)18 * cin * coutp;
+// bf16x3: the same layout twice -- dst[0, n) = bf16_rn(w), dst[n, 2n) = bf16_rn(w - bf16_rn(w)), n = 9 cin coutp; no saturation.
+__global__ void conv2d_pack_bf16x3_kernel(const float* __restrict__ w, int cin, int cout, int coutp, __nv_bfloat16* __restrict__ dst) {
+    const int total = 9 * cin * coutp;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+        const int e = i & 7;
+        const int row = (i >> 3) % (3 * coutp);
+        const int half = (i / (8 * 3 * coutp)) & 1;
+        const int blk = i / (16 * 3 * coutp);
+        const int kx = blk % 3, c16 = blk / 3;
+        const int kyb = row / coutp, co = row - kyb * coutp;
+        const int ci = c16 * 16 + half * 8 + e;
+        float v = 0.0f;
+        if (co < cout) v = w[(((size_t)co * cin + ci) * 3 + (2 - kyb)) * 3 + kx];
+        const __nv_bfloat16 hi = __float2bfloat16_rn(v);
+        dst[i] = hi;
+        dst[total + i] = __float2bfloat16_rn(v - __bfloat162float(hi));
+    }
 }
 
-extern "C" int effimvs_conv2d_tf32_supported(int cin, int cout) {
+int pow2_cols(int n) { int c = 32; while (c < n) c <<= 1; return c; }
+// channels per K phase: the whole input when it is 16, 32 or 64 channels, else 32- or 16-channel phases; bf16x3 (a stage holds
+// two copies): at most 32
+int phase_channels(int cin) { return (cin == 16 || cin == 32 || cin == 64) ? cin : (cin % 32 == 0 ? 32 : 16); }
+int phase_channels(int cin, int prec) { return prec == C2_BF16X3 ? (cin % 32 == 0 ? 32 : 16) : phase_channels(cin); }
+// copies of each operand: the bf16x3 weight image and staged rows hold hi and lo
+int operand_copies(int prec) { return prec == C2_BF16X3 ? 2 : 1; }
+
+size_t packed_bytes(int cin, int cout, int prec) {
+    if (cin <= 0 || cout <= 0) return 0;
+    const int coutp = (cout + 15) / 16 * 16;
+    return (size_t)18 * operand_copies(prec) * cin * coutp;
+}
+
+int supported(int cin, int cout, int prec) {
     if (cin < 16 || cin % 16 != 0 || cout < 4 || cout % 4 != 0 || cout > C2_MAX_COUT) return 0;
     const int coutp = (cout + 15) / 16 * 16;
-    const int kc = phase_channels(cin);
-    const size_t smem = (size_t)18 * cin * coutp + (size_t)3 * (kc / 8) * C2_CG_BYTES + C2_EPI_BYTES;
+    const int kc = phase_channels(cin, prec);
+    const size_t smem = packed_bytes(cin, cout, prec) + (size_t)3 * operand_copies(prec) * (kc / 8) * C2_CG_BYTES + C2_EPI_BYTES;
     if (smem > 224 * 1024) return 0;
     if (4 * coutp > 512) return 0;
     return 1;
 }
 
-extern "C" int effimvs_conv2d_tf32_pack(const float* w, int cin, int cout, void* packed, void* stream) {
-    EFFI_REQUIRE(w && packed, EFFIMVS_EINVAL, "conv2d_tf32_pack: null pointer");
-    EFFI_REQUIRE(effimvs_conv2d_tf32_supported(cin, cout), EFFIMVS_EUNSUPPORTED, "conv2d_tf32_pack: cin=%d cout=%d not supported", cin, cout);
+int pack(const char* name, int prec, const float* w, int cin, int cout, void* packed, void* stream) {
+    EFFI_REQUIRE(w && packed, EFFIMVS_EINVAL, "%s: null pointer", name);
+    EFFI_REQUIRE(supported(cin, cout, prec), EFFIMVS_EUNSUPPORTED, "%s: cin=%d cout=%d not supported", name, cin, cout);
     const int coutp = (cout + 15) / 16 * 16;
     const int total = 9 * cin * coutp;
-    conv2d_pack_kernel<<<std::min(ceil_div(total, 256), 1024), 256, 0, (cudaStream_t)stream>>>(w, cin, cout, coutp, (__half*)packed);
+    const int grid = std::min(ceil_div(total, 256), 1024);
+    if (prec == C2_BF16X3) {
+        conv2d_pack_bf16x3_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(w, cin, cout, coutp, (__nv_bfloat16*)packed);
+        return check_launch("conv2d_pack_bf16x3_kernel");
+    }
+    conv2d_pack_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(w, cin, cout, coutp, (__half*)packed);
     return check_launch("conv2d_pack_kernel");
 }
 
-extern "C" int effimvs_conv2d_tf32(const float* in0, long long in0_ps, int c0, const float* in1, long long in1_ps, int c1,
-                                   const void* packed, const float* bias, int cout, int B, int H, int W, int mode,
-                                   float* out, long long out_ps, const float* aux0, long long aux0_ps, float* aux1,
-                                   long long aux1_ps, void* stream) {
-    EFFI_REQUIRE(in0 && packed && out, EFFIMVS_EINVAL, "conv2d_tf32: null pointer");
-    EFFI_REQUIRE(B > 0 && H >= 2 && W >= 1, EFFIMVS_EINVAL, "conv2d_tf32: bad shape %dx%dx%d", B, H, W);
-    EFFI_REQUIRE(c0 > 0 && c0 % 8 == 0 && c1 >= 0 && c1 % 8 == 0 && (c1 == 0 || in1), EFFIMVS_EINVAL, "conv2d_tf32: bad channel segments %d + %d", c0, c1);
+long long* g_conv2d_timeline = nullptr;
+
+// the host side of both families: validation, budgets and the launch of the instantiation for (mode, K phase, precision)
+int launch(const char* name, int prec, const float* in0, long long in0_ps, int c0, const float* in1, long long in1_ps, int c1,
+           const void* packed, const float* bias, int cout, int B, int H, int W, int mode,
+           float* out, long long out_ps, const float* aux0, long long aux0_ps, float* aux1,
+           long long aux1_ps, void* stream) {
+    EFFI_REQUIRE(in0 && packed && out, EFFIMVS_EINVAL, "%s: null pointer", name);
+    EFFI_REQUIRE(B > 0 && H >= 2 && W >= 1, EFFIMVS_EINVAL, "%s: bad shape %dx%dx%d", name, B, H, W);
+    EFFI_REQUIRE(c0 > 0 && c0 % 8 == 0 && c1 >= 0 && c1 % 8 == 0 && (c1 == 0 || in1), EFFIMVS_EINVAL, "%s: bad channel segments %d + %d", name, c0, c1);
     const int cin = c0 + c1;
-    EFFI_REQUIRE(effimvs_conv2d_tf32_supported(cin, cout), EFFIMVS_EUNSUPPORTED, "conv2d_tf32: cin=%d cout=%d not supported", cin, cout);
-    EFFI_REQUIRE(mode >= EFFIMVS_CONV2D_BIAS && mode <= EFFIMVS_CONV2D_GRU_UPDATE, EFFIMVS_EINVAL, "conv2d_tf32: bad mode %d", mode);
+    EFFI_REQUIRE(supported(cin, cout, prec), EFFIMVS_EUNSUPPORTED, "%s: cin=%d cout=%d not supported", name, cin, cout);
+    EFFI_REQUIRE(mode >= EFFIMVS_CONV2D_BIAS && mode <= EFFIMVS_CONV2D_GRU_UPDATE, EFFIMVS_EINVAL, "%s: bad mode %d", name, mode);
     EFFI_REQUIRE(in0_ps >= c0 && in0_ps % 8 == 0 && (c1 == 0 || (in1_ps >= c1 && in1_ps % 8 == 0)) && out_ps % 4 == 0,
-                 EFFIMVS_EINVAL, "conv2d_tf32: input pixel strides must be multiples of 8 floats, the output's of 4");
+                 EFFIMVS_EINVAL, "%s: input pixel strides must be multiples of 8 floats, the output's of 4", name);
     EFFI_REQUIRE((((uintptr_t)in0 | (uintptr_t)in1) & 31) == 0 && (((uintptr_t)out | (uintptr_t)aux0 | (uintptr_t)aux1 | (uintptr_t)packed) & 15) == 0,
-                 EFFIMVS_EINVAL, "conv2d_tf32: input maps must be 32-byte aligned, the other pointers 16-byte aligned");
-    EFFI_REQUIRE((long long)W * in0_ps < (1ll << 31) && (long long)W * in1_ps < (1ll << 31), EFFIMVS_EUNSUPPORTED, "conv2d_tf32: a row of a map must be below 2^31 floats");
-    if (mode == EFFIMVS_CONV2D_ADD_RELU) EFFI_REQUIRE(aux0 && aux0_ps % 4 == 0, EFFIMVS_EINVAL, "conv2d_tf32: ADD_RELU needs the addend map");
+                 EFFIMVS_EINVAL, "%s: input maps must be 32-byte aligned, the other pointers 16-byte aligned", name);
+    EFFI_REQUIRE((long long)W * in0_ps < (1ll << 31) && (long long)W * in1_ps < (1ll << 31), EFFIMVS_EUNSUPPORTED, "%s: a row of a map must be below 2^31 floats", name);
+    if (mode == EFFIMVS_CONV2D_ADD_RELU) EFFI_REQUIRE(aux0 && aux0_ps % 4 == 0, EFFIMVS_EINVAL, "%s: ADD_RELU needs the addend map", name);
     if (mode == EFFIMVS_CONV2D_GRU_GATES)
         EFFI_REQUIRE(aux0 && aux1 && bias && cout % 32 == 0 && aux0_ps % 4 == 0 && aux1_ps % 4 == 0, EFFIMVS_EINVAL,
-                     "conv2d_tf32: GRU_GATES needs h_prev, the z buffer, the bias and cout = 2h with h a multiple of 16");
-    if (mode == EFFIMVS_CONV2D_GRU_UPDATE) EFFI_REQUIRE(aux0 && bias && aux0_ps % 4 == 0, EFFIMVS_EINVAL, "conv2d_tf32: GRU_UPDATE needs z and the bias");
+                     "%s: GRU_GATES needs h_prev, the z buffer, the bias and cout = 2h with h a multiple of 16", name);
+    if (mode == EFFIMVS_CONV2D_GRU_UPDATE) EFFI_REQUIRE(aux0 && bias && aux0_ps % 4 == 0, EFFIMVS_EINVAL, "%s: GRU_UPDATE needs z and the bias", name);
 
     C2Params P;
     P.in0 = in0; P.ps0 = in0_ps; P.c0 = c0;
     P.in1 = in1 ? in1 : in0; P.ps1 = in1 ? in1_ps : in0_ps; P.c1 = c1;
     P.cin = cin; P.cout = cout; P.coutp = (cout + 15) / 16 * 16;
     P.B = B; P.H = H; P.W = W;
-    P.kc = phase_channels(cin);
+    P.kc = phase_channels(cin, prec);
     P.n_phases = cin / P.kc;
     P.mode = mode;
     P.tl = g_conv2d_timeline;
@@ -717,8 +781,8 @@ extern "C" int effimvs_conv2d_tf32(const float* in0, long long in0_ps, int c0, c
     P.out = out; P.out_ps = out_ps;
     P.aux0 = aux0; P.aux0_ps = aux0_ps;
     P.aux1 = aux1; P.aux1_ps = aux1_ps;
-    P.w_bytes = 18 * cin * P.coutp;
-    P.stage_bytes = (P.kc / 8) * C2_CG_BYTES;
+    P.w_bytes = (int)packed_bytes(cin, cout, prec);
+    P.stage_bytes = operand_copies(prec) * (P.kc / 8) * C2_CG_BYTES;
     // CTAs per SM: three 288-thread CTAs (two producer warps per group) when shared memory, registers and TMEM allow -- every
     // role of this kernel is a chain of per-row latencies, so resident CTAs are what fills the SM --, else two or one
     // 416-thread CTAs.  The accumulator ring takes the TMEM columns that is left per CTA (the fewer wrap-arounds, the fewer
@@ -750,21 +814,56 @@ extern "C" int effimvs_conv2d_tf32(const float* in0, long long in0_ps, int c0, c
     P.n_units = B * P.strips * P.chunks;
 
     typedef void (*KernelFn)(C2Params, const uint8_t*);
-#define C2_ROW(M) {conv2d_tc_kernel<M, 2>, conv2d_tc_kernel<M, 4>, conv2d_tc_kernel<M, 8>}
-    static const KernelFn table[5][3] = {C2_ROW(EFFIMVS_CONV2D_BIAS), C2_ROW(EFFIMVS_CONV2D_BIAS_RELU), C2_ROW(EFFIMVS_CONV2D_ADD_RELU),
-                                         C2_ROW(EFFIMVS_CONV2D_GRU_GATES), C2_ROW(EFFIMVS_CONV2D_GRU_UPDATE)};
+#define C2_ROW(M) {{conv2d_tc_kernel<M, 2, C2_F16>, conv2d_tc_kernel<M, 4, C2_F16>, conv2d_tc_kernel<M, 8, C2_F16>}, \
+                   {conv2d_tc_kernel<M, 2, C2_BF16X3>, conv2d_tc_kernel<M, 4, C2_BF16X3>, nullptr}}
+    static const KernelFn table[5][2][3] = {C2_ROW(EFFIMVS_CONV2D_BIAS), C2_ROW(EFFIMVS_CONV2D_BIAS_RELU), C2_ROW(EFFIMVS_CONV2D_ADD_RELU),
+                                            C2_ROW(EFFIMVS_CONV2D_GRU_GATES), C2_ROW(EFFIMVS_CONV2D_GRU_UPDATE)};
 #undef C2_ROW
     const int gi = P.kc == 16 ? 0 : (P.kc == 32 ? 1 : 2);
-    const KernelFn fn = table[mode][gi];
-    static bool attr_set[64][5][3] = {};   // per device and instantiation; idempotent, a race only repeats the call
+    const KernelFn fn = table[mode][prec][gi];      // (bf16x3 phases are at most 32 channels: gi < 2)
+    static bool attr_set[64][5][2][3] = {};   // per device and instantiation; idempotent, a race only repeats the call
     int dev = 0;
     cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev][mode][gi]) {
+    if (dev < 0 || dev >= 64 || !attr_set[dev][mode][prec][gi]) {
         cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024);
-        EFFI_REQUIRE(e == cudaSuccess, EFFIMVS_ECUDA, "conv2d_tf32: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-        if (dev >= 0 && dev < 64) attr_set[dev][mode][gi] = true;
+        EFFI_REQUIRE(e == cudaSuccess, EFFIMVS_ECUDA, "%s: cudaFuncSetAttribute: %s", name, cudaGetErrorString(e));
+        if (dev >= 0 && dev < 64) attr_set[dev][mode][prec][gi] = true;
     }
     launch_kernel(fn, dim3(std::min(G, P.n_units)), dim3((C2_PROD_WARP0 + C2_PROD_GROUPS * P.gw) * 32), smem, (cudaStream_t)stream, P,
                   (const uint8_t*)packed);
     return check_launch("conv2d_tc_kernel");
+}
+
+}  // namespace
+}  // namespace effimvs
+
+using namespace effimvs;
+
+/* profiling hook (not part of include/effimvs.h): device buffer of 3 * 64 * 4 int64 that CTA 0 of the following launches fills */
+extern "C" void effimvs_conv2d_debug_timeline(void* buf) { g_conv2d_timeline = (long long*)buf; }
+
+extern "C" size_t effimvs_conv2d_tf32_packed_bytes(int cin, int cout) { return packed_bytes(cin, cout, C2_F16); }
+extern "C" int effimvs_conv2d_tf32_supported(int cin, int cout) { return supported(cin, cout, C2_F16); }
+extern "C" int effimvs_conv2d_tf32_pack(const float* w, int cin, int cout, void* packed, void* stream) {
+    return pack("conv2d_tf32_pack", C2_F16, w, cin, cout, packed, stream);
+}
+extern "C" int effimvs_conv2d_tf32(const float* in0, long long in0_ps, int c0, const float* in1, long long in1_ps, int c1,
+                                   const void* packed, const float* bias, int cout, int B, int H, int W, int mode,
+                                   float* out, long long out_ps, const float* aux0, long long aux0_ps, float* aux1,
+                                   long long aux1_ps, void* stream) {
+    return launch("conv2d_tf32", C2_F16, in0, in0_ps, c0, in1, in1_ps, c1, packed, bias, cout, B, H, W, mode, out, out_ps,
+                  aux0, aux0_ps, aux1, aux1_ps, stream);
+}
+
+extern "C" size_t effimvs_conv2d_bf16x3_packed_bytes(int cin, int cout) { return packed_bytes(cin, cout, C2_BF16X3); }
+extern "C" int effimvs_conv2d_bf16x3_supported(int cin, int cout) { return supported(cin, cout, C2_BF16X3); }
+extern "C" int effimvs_conv2d_bf16x3_pack(const float* w, int cin, int cout, void* packed, void* stream) {
+    return pack("conv2d_bf16x3_pack", C2_BF16X3, w, cin, cout, packed, stream);
+}
+extern "C" int effimvs_conv2d_bf16x3(const float* in0, long long in0_ps, int c0, const float* in1, long long in1_ps, int c1,
+                                     const void* packed, const float* bias, int cout, int B, int H, int W, int mode,
+                                     float* out, long long out_ps, const float* aux0, long long aux0_ps, float* aux1,
+                                     long long aux1_ps, void* stream) {
+    return launch("conv2d_bf16x3", C2_BF16X3, in0, in0_ps, c0, in1, in1_ps, c1, packed, bias, cout, B, H, W, mode, out, out_ps,
+                  aux0, aux0_ps, aux1, aux1_ps, stream);
 }

@@ -8,6 +8,7 @@ libeffimvs.so is missing the import of ``capi`` raises.
 from __future__ import annotations
 
 import collections
+import functools
 import os
 import weakref
 
@@ -104,7 +105,7 @@ class CudaHotPath:
     fused_update = True      # net.UpdateBlock.forward_fused: GRU / upsampling glue kernels (SURVEY section 8(f) row 3)
 
     def __init__(self, precision: str = "f32", native_projection: bool = False, persistent_workspaces: bool = True,
-                 parallel_branches: bool = False):
+                 parallel_branches: bool = False, conv2d_precision=None):
         """precision of the 3-D regularization: 'f32' (CUDA-core direct convs), 'bf16' (tcgen05 implicit
         GEMM, one bf16 MMA per product) or 'bf16x3' (tcgen05, hi/lo split operands, fp32-grade).
         native_projection: compute P_src @ inverse(P_ref) with the library's fp64 kernel instead
@@ -115,7 +116,11 @@ class CudaHotPath:
         parallel_branches: offer a side stream for the independent cross-scale branches (net.EffiMVSPlus).  Off by
         default: measured on B200 the forked graph is slower (7.00 vs 6.91 ms per DTU depth map) -- the persistent
         tensor-core kernels of the two branches cannot co-reside, and the fork / join costs more than the small
-        CUDA-core layers gain."""
+        CUDA-core layers gain.
+        conv2d_precision: arithmetic of the update block's tensor-core 3x3 convolutions (csrc/conv2d_tc.cu).  None: operands
+        rounded to fp16 (TF32's 11 significant bits), used only while torch.backends.cudnn.allow_tf32 is on -- with it off
+        those layers stay on cuDNN's fp32 kernels.  'bf16x3': operands as hi + lo bf16 pairs, three products, fp32
+        accumulation and range (~2^-16 relative, fp32-grade), so the kernel also runs with allow_tf32 off."""
         self.precision = {"f32": capi.PREC_F32, "bf16": capi.PREC_BF16, "bf16x3": capi.PREC_BF16X3}[precision]
         self.native_projection = native_projection
         self.persistent_workspaces = persistent_workspaces and os.environ.get("EFFIMVS_PERSISTENT_WS", "1") != "0"
@@ -124,6 +129,16 @@ class CudaHotPath:
         self._workspaces = _WorkspaceCache()
         self._side_streams = {}
         self._tracked = set()
+        if conv2d_precision not in (None, "bf16x3"):
+            raise ValueError("conv2d_precision must be None or 'bf16x3', got {!r}".format(conv2d_precision))
+        if conv2d_precision == "bf16x3":
+            # the table's conv2d_tc* entries bound to the bf16x3 kernel; net.py keys its packed weight images by
+            # conv2d_precision and runs fp32-grade convolutions whatever allow_tf32 says
+            self.conv2d_precision = "bf16x3"
+            self.conv2d_fp32_grade = True
+            self.conv2d_tc = functools.partial(ops.conv2d_tc, precision="bf16x3")
+            self.conv2d_tc_pack = functools.partial(ops.conv2d_tc_pack, precision="bf16x3")
+            self.conv2d_tc_supported = functools.partial(ops.conv2d_tc_supported, precision="bf16x3")
 
     def side_stream(self, device):
         """Stream for work that is independent of the caller's current stream (None: run it in line)."""
@@ -289,7 +304,10 @@ class CudaHotPath:
     encoder_tail_ctx = staticmethod(ops.encoder_tail_ctx)
     gru_init = staticmethod(ops.gru_init)
     gru_init_ctx = staticmethod(ops.gru_init_ctx)
-    # the block's 3x3 convolutions on the tensor cores, gate arithmetic as epilogues (csrc/conv2d_tc.cu)
+    # the block's 3x3 convolutions on the tensor cores, gate arithmetic as epilogues (csrc/conv2d_tc.cu); fp16 operands unless
+    # the instance was built with conv2d_precision='bf16x3'
+    conv2d_precision = "f16"
+    conv2d_fp32_grade = False
     conv2d_tc = staticmethod(ops.conv2d_tc)
     conv2d_tc_pack = staticmethod(ops.conv2d_tc_pack)
     conv2d_tc_supported = staticmethod(ops.conv2d_tc_supported)

@@ -339,12 +339,14 @@ def _conv_tc_enabled(glue, h, H, W):
     """Whether the update block's 3x3 convolutions run on the library's tensor-core kernel (csrc/conv2d_tc.cu: operands with
     the 11 significant bits of TF32, fp32 accumulation, gate arithmetic as epilogues) instead of cuDNN.  Follows PyTorch's own
     switch for that arithmetic class: with torch.backends.cudnn.allow_tf32 = False (fp32 products wanted) cuDNN's fp32 kernels
-    stay.  EFFIMVS_CONV2D = 0 / 1 forces it off / on; by default maps below EFFIMVS_CONV2D_MIN_PIXELS pixels (the 1/8-resolution
-    stage, where launch and prologue latency dominate and cuDNN is faster) stay on cuDNN as well."""
+    stay -- unless the glue's convolutions are fp32-grade (glue.conv2d_fp32_grade: CudaHotPath(conv2d_precision='bf16x3'), hi/lo
+    bf16 operands), which run either way.  EFFIMVS_CONV2D = 0 / 1 forces it off / on; by default maps below
+    EFFIMVS_CONV2D_MIN_PIXELS pixels (the 1/8-resolution stage, where launch and prologue latency dominate and cuDNN is faster)
+    stay on cuDNN as well."""
     env = os.environ.get("EFFIMVS_CONV2D", "auto")
     if env == "0" or not hasattr(glue, "conv2d_tc") or h % 16 != 0:
         return False
-    if env != "1" and not torch.backends.cudnn.allow_tf32:
+    if env != "1" and not torch.backends.cudnn.allow_tf32 and not getattr(glue, "conv2d_fp32_grade", False):
         return False
     sup = glue.conv2d_tc_supported
     if not (sup(2 * h, 2 * h) and sup(2 * h, h) and sup(h, h) and sup(h, 2 * h)):
@@ -354,8 +356,10 @@ def _conv_tc_enabled(glue, h, H, W):
 
 def _tc_update_weights(block, glue, w):
     """Packed weight images of the block's six 3x3 convolutions for conv2d_tc, built once per weight set (they live in the
-    dict _fused_update_weights caches, so they are rebuilt when a parameter changes)."""
-    tc = w.get("tc")
+    dict _fused_update_weights caches, so they are rebuilt when a parameter changes).  Keyed by the glue's operand precision:
+    one model may run under hot paths of different precisions, and each kernel reads only its own image format."""
+    key = ("tc", getattr(glue, "conv2d_precision", "f16"))
+    tc = w.get(key)
     if tc is None:
         g, e, hd = block.depth_gru, block.encoder, block.depth_head
         hm = e.convd.out_channels
@@ -365,7 +369,7 @@ def _tc_update_weights(block, glue, w):
               "zr": glue.conv2d_tc_pack(w["wzr"]), "q": glue.conv2d_tc_pack(g.convq.weight.detach()),
               "head1": glue.conv2d_tc_pack(hd.conv1.weight.detach()), "mask0": glue.conv2d_tc_pack(block.mask[0].weight.detach()),
               "b_zr": torch.cat([g.convz.bias.detach(), g.convr.bias.detach()]).contiguous()}
-        w["tc"] = tc
+        w[key] = tc
     return tc
 
 

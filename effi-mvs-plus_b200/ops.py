@@ -888,8 +888,20 @@ def encoder_tail_ctx(m: Tensor, w_m: Tensor, ctx: Tensor, ctx_offset: int, cx: i
 
 # -------------------------------------------------------------------------------------------
 # SURVEY section 8(f) row 3, the convolutions: 3x3 convolutions of the update block on the tensor cores (csrc/conv2d_tc.cu)
-def conv2d_tc_supported(cin: int, cout: int) -> bool:
-    return bool(_lib.effimvs_conv2d_tf32_supported(int(cin), int(cout)))
+# precision "f16": operands rounded to fp16 (TF32's 11 significant bits, saturating at +-65504), the effimvs_conv2d_tf32 family;
+# "bf16x3": operands as hi + lo bf16 pairs, three products, fp32 range (fp32-grade), the effimvs_conv2d_bf16x3 family
+def _conv2d_fns(precision: str):
+    if precision == "f16":
+        return (_lib.effimvs_conv2d_tf32_supported, _lib.effimvs_conv2d_tf32_packed_bytes, _lib.effimvs_conv2d_tf32_pack,
+                _lib.effimvs_conv2d_tf32)
+    if precision == "bf16x3":
+        return (_lib.effimvs_conv2d_bf16x3_supported, _lib.effimvs_conv2d_bf16x3_packed_bytes, _lib.effimvs_conv2d_bf16x3_pack,
+                _lib.effimvs_conv2d_bf16x3)
+    raise ValueError("conv2d_tc: precision must be 'f16' or 'bf16x3', got {!r}".format(precision))
+
+
+def conv2d_tc_supported(cin: int, cout: int, precision: str = "f16") -> bool:
+    return bool(_conv2d_fns(precision)[0](int(cin), int(cout)))
 
 
 def _cl_view(t: Tensor, name: str):
@@ -906,30 +918,35 @@ def _cl_view(t: Tensor, name: str):
 
 @torch.library.custom_op("effimvs::conv2d_tc_pack", mutates_args=())
 @_on_tensor_device
-def conv2d_tc_pack(weight: Tensor) -> Tensor:
-    """(cout, cin, 3, 3) fp32 -> the kernel's packed fp16 weight image (once per weight tensor)."""
+def conv2d_tc_pack(weight: Tensor, precision: str = "f16") -> Tensor:
+    """(cout, cin, 3, 3) fp32 -> the kernel's packed weight image for `precision` (once per weight tensor): fp16, or the
+    bf16 hi image followed by the lo image for "bf16x3"."""
+    supported, packed_bytes, pack, _ = _conv2d_fns(precision)
     weight = _dev(weight, "conv2d_tc_pack")
     cout, cin = weight.shape[:2]
-    if tuple(weight.shape[2:]) != (3, 3) or not conv2d_tc_supported(cin, cout):
-        raise ValueError("conv2d_tc_pack: unsupported weight shape {}".format(tuple(weight.shape)))
-    packed = torch.empty(_lib.effimvs_conv2d_tf32_packed_bytes(cin, cout) // 4, device=weight.device, dtype=torch.float32)
+    if tuple(weight.shape[2:]) != (3, 3) or not supported(cin, cout):
+        raise ValueError("conv2d_tc_pack: unsupported weight shape {} for precision {}".format(tuple(weight.shape), precision))
+    packed = torch.empty(packed_bytes(cin, cout) // 4, device=weight.device, dtype=torch.float32)
     _count(1)
-    capi.check(_lib.effimvs_conv2d_tf32_pack(weight.data_ptr(), cin, cout, packed.data_ptr(), _stream()))
+    capi.check(pack(weight.data_ptr(), cin, cout, packed.data_ptr(), _stream()))
     return packed
 
 
 @conv2d_tc_pack.register_fake
-def _(weight):
-    return weight.new_empty(9 * weight.shape[1] * ((weight.shape[0] + 15) // 16 * 16) // 2)
+def _(weight, precision="f16"):
+    copies = 2 if precision == "bf16x3" else 1
+    return weight.new_empty(copies * 9 * weight.shape[1] * ((weight.shape[0] + 15) // 16 * 16) // 2)
 
 
 @torch.library.custom_op("effimvs::conv2d_tc", mutates_args=("out", "aux1"))
 @_on_tensor_device
 def conv2d_tc(in0: Tensor, in1: Optional[Tensor], packed: Tensor, bias: Optional[Tensor], cout: int, mode: int, out: Tensor,
-              aux0: Optional[Tensor], aux1: Optional[Tensor]) -> None:
+              aux0: Optional[Tensor], aux1: Optional[Tensor], precision: str = "f16") -> None:
     """3x3 / stride 1 / padding 1 convolution of cat[in0, in1] (channels-last maps or channel slices of such maps, read and
     written in place) with the epilogue `mode` (capi.CONV2D_*): BIAS / BIAS_RELU -> out; ADD_RELU: out = relu(acc + aux0);
-    GRU_GATES: aux1 = z, out = r * aux0 (aux0 = h); GRU_UPDATE: out = (1 - aux0) * out + aux0 * tanh(acc + bias) (aux0 = z)."""
+    GRU_GATES: aux1 = z, out = r * aux0 (aux0 = h); GRU_UPDATE: out = (1 - aux0) * out + aux0 * tanh(acc + bias) (aux0 = z).  `packed` from conv2d_tc_pack with the same
+    precision."""
+    _, packed_bytes, _, conv = _conv2d_fns(precision)
     B, c0, H, W = in0.shape
     p0, ps0 = _cl_view(in0, "in0")
     p1, ps1, c1 = None, 0, 0
@@ -947,16 +964,16 @@ def conv2d_tc(in0: Tensor, in1: Optional[Tensor], packed: Tensor, bias: Optional
     for a in (aux0, aux1):
         if a is not None and tuple(a.shape) != (B, h, H, W):
             raise ValueError("conv2d_tc: aux map {} should be {}".format(tuple(a.shape), (B, h, H, W)))
-    if packed.numel() * 4 != _lib.effimvs_conv2d_tf32_packed_bytes(c0 + c1, cout):
-        raise ValueError("conv2d_tc: packed weights do not match cin = {} cout = {}".format(c0 + c1, cout))
+    if packed.numel() * 4 != packed_bytes(c0 + c1, cout):
+        raise ValueError("conv2d_tc: packed weights do not match cin = {} cout = {} ({})".format(c0 + c1, cout, precision))
     bias = _dev(bias, "conv2d_tc") if bias is not None else None
     _count(1)
-    capi.check(_lib.effimvs_conv2d_tf32(p0, ps0, c0, p1, ps1, c1, packed.data_ptr(), _opt(bias), cout, B, H, W, mode,
-                                        po, pso, pa0, psa0, pa1, psa1, _stream()))
+    capi.check(conv(p0, ps0, c0, p1, ps1, c1, packed.data_ptr(), _opt(bias), cout, B, H, W, mode,
+                    po, pso, pa0, psa0, pa1, psa1, _stream()))
 
 
 @conv2d_tc.register_fake
-def _(in0, in1, packed, bias, cout, mode, out, aux0, aux1):
+def _(in0, in1, packed, bias, cout, mode, out, aux0, aux1, precision="f16"):
     return None
 
 

@@ -355,6 +355,20 @@ int effimvs_conv2d_tf32(const float* in0, long long in0_pixstride, int c0, const
                         float* out, long long out_pixstride, const float* aux0, long long aux0_pixstride,
                         float* aux1, long long aux1_pixstride, void* stream);
 
+/* The same convolutions with fp32-grade arithmetic (bf16x3), the class of the 3-D nets' default mode: every operand, input
+ * and weight, is carried as hi = bf16(x) and lo = bf16(x - hi) (together ~2^-16 relative), and each product is formed as
+ * hi*hi + hi*lo + lo*hi with fp32 accumulation.  Range: fp32's -- nothing saturates.  The packed image is the hi weights
+ * followed by the lo weights: 36 * cin * roundup(cout, 16) bytes.  Arguments, modes, layouts and error codes as the
+ * _tf32 family above.  Both weight images and a two-copy input ring live in shared memory, so fewer shapes are supported:
+ * up to 64 x 64 channels (the update block at hidden sizes 16 and 32), not 96 x 96. */
+int effimvs_conv2d_bf16x3_supported(int cin, int cout);
+size_t effimvs_conv2d_bf16x3_packed_bytes(int cin, int cout);
+int effimvs_conv2d_bf16x3_pack(const float* w, int cin, int cout, void* packed, void* stream);
+int effimvs_conv2d_bf16x3(const float* in0, long long in0_pixstride, int c0, const float* in1, long long in1_pixstride, int c1,
+                          const void* packed, const float* bias, int cout, int B, int H, int W, int mode,
+                          float* out, long long out_pixstride, const float* aux0, long long aux0_pixstride,
+                          float* aux1, long long aux1_pixstride, void* stream);
+
 /* ---- SURVEY section 8(f) row 2: the DTU pipeline's NumPy / cv2.remap geometric filter ------------------------
  * reproject_with_depth + check_geometric_consistency + the aggregation of filter_depth
  * (test_dtu_dypcd.py:164-233, 261-309, 320-337) for one reference view in one kernel.
