@@ -4,7 +4,7 @@ collective during depth inference, ONE all-gather of the final depth maps before
 """
 from __future__ import annotations
 
-from typing import Callable, Dict, List, Sequence
+from typing import Callable, Dict, List, Sequence, Tuple
 
 import torch
 import torch.distributed as dist
@@ -37,6 +37,19 @@ def view_slot(i: int, n_views: int, world: int, mode: str = "round_robin"):
     q, r = divmod(n_views, world)
     owner = i // (q + 1) if i < r * (q + 1) else r + (i - r * (q + 1)) // max(q, 1)
     return owner, i - block_start(n_views, owner, world)
+
+
+def view_groups(views: Sequence, k: int) -> List[Tuple[list, int]]:
+    """`views` in order as consecutive groups of k, each with the number of its real entries: a short last group is padded
+    to k entries with copies of its last entry (whose results the caller drops).  No views give no groups."""
+    if k < 1:
+        raise ValueError("groups of at least one view, got k = {}".format(k))
+    views = list(views)
+    out = []
+    for a in range(0, len(views), k):
+        g = views[a:a + k]
+        out.append((g + [g[-1]] * (k - len(g)), len(g)))
+    return out
 
 
 def gather_depths(local: Dict[int, torch.Tensor], n_views: int, rank: int, world: int, h: int, w: int, device,
@@ -78,23 +91,35 @@ def agree_on_size(local_hw, n_views: int, world: int, device):
 
 @torch.no_grad()
 def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Sequence[int]], rank: int = 0, world: int = 1,
-              device="cuda", fuse_pairs: Sequence[Sequence[int]] = None, timings: dict = None, sharding: str = "round_robin"):
+              device="cuda", fuse_pairs: Sequence[Sequence[int]] = None, timings: dict = None, sharding: str = "round_robin",
+              views_per_batch: int = None):
     """infer(ref_view, src_views) -> (depth (h,w), conf (hc,wc)) on `device`;
     fuse(ref_view, ref_depth (1,1,h,w), conf (1,hc,wc), src_views, src_depths (1,v,1,h,w)) -> dict with
     'final' (1,1,h,w) bool and 'points' (1,3,h,w).
     pairs[i]: source views used for the depth map of view i; fuse_pairs[i] (default: pairs[i]): source
     views whose depth maps the consistency filter of view i reads (upstream: 4 and up to 10).
+    When infer has `batch` (infer.batch([(ref_view, src_views), ...]) -> [(depth, conf), ...]), the rank's views go to
+    it in view order, in groups of at most views_per_batch (default: infer.views_per_batch, else 1).
     Returns {ref_view: (points (k,3), depth (h,w))} for the views this rank owns."""
     fuse_pairs = pairs if fuse_pairs is None else fuse_pairs
     mine = shard_views(n_views, rank, world, sharding)
+    batch = getattr(infer, "batch", None)
+    k = views_per_batch if views_per_batch is not None else getattr(infer, "views_per_batch", 1)
+    if batch is None and k != 1:
+        raise ValueError("views_per_batch = {} needs an infer with a `batch` method".format(k))
     depths, confs = {}, {}
     timed = timings is not None and torch.cuda.is_available() and str(device).startswith("cuda")
     if timed:
         ev_start = torch.cuda.Event(enable_timing=True)
         ev_start.record()
-    for i in mine:
-        d, c = infer(i, list(pairs[i]))
-        depths[i], confs[i] = d, c
+    if batch is None:
+        for i in mine:
+            depths[i], confs[i] = infer(i, list(pairs[i]))
+    else:
+        for group, n in view_groups(mine, k):
+            real = group[:n]
+            for i, (d, c) in zip(real, batch([(i, list(pairs[i])) for i in real])):
+                depths[i], confs[i] = d, c
     # a rank without a view (n_views < world) still enters the collective below with a zero block
     h, w = agree_on_size(tuple(next(iter(depths.values())).shape[-2:]) if depths else None, n_views, world, device)
     ev = None
@@ -124,91 +149,146 @@ def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Seq
     return out
 
 
-class GraphedViewRunner:
-    """Depth inference of one reference view from cached feature pyramids as two CUDA graphs: `encode` (one image
-    through the FPN) and `forward` (the cascade on static feature / camera buffers).  The hot path has no host
-    synchronisation, so both capture; per view the host only issues a handful of device-to-device copies and
-    one replay instead of ~320 launches (section 8(f) row 1 + SURVEY section 8(e) "CUDA-graph the forward")."""
+def _as_words(*ts):
+    """contiguous (N, ...) tensors as (N, row) matrices of 16-byte complex128 words when every row allows it, else of their
+    own elements: index_select / index_copy_ along dim 0 then move 16 bytes per element instead of 4 (with 4-byte elements
+    the 49-view DTU scene at one view per replay was 1.4 % slower than plain per-view copies).  The bits are copied, never
+    computed on."""
+    flat = [t.view(t.shape[0], -1) for t in ts]
+    if all((f.shape[1] * f.element_size()) % 16 == 0 and f.data_ptr() % 16 == 0 for f in flat):
+        return [f.view(torch.complex128) for f in flat]
+    return flat
 
-    def __init__(self, model, imgs: torch.Tensor, cams: Dict[str, torch.Tensor], depth_values: torch.Tensor, n_src: int):
+
+class GraphedViewRunner:
+    """Depth inference of reference views from a per-scene feature cache as two CUDA graphs: `encode` (one image through
+    the FPN into its rows of the cache) and `forward` (the cascade for `views_per_replay` = K reference views at once).
+    The hot path has no host synchronisation, so both capture; per K views the host issues one device-to-device index
+    copy and one replay instead of ~320 launches per view (section 8(f) row 1 + SURVEY section 8(e) "CUDA-graph the
+    forward").  Batching fills the launches of the 1/8-resolution stage, which one view leaves mostly idle.
+
+    The cache is one preallocated tensor per stage, (N_images, h, w, C) in memory: row j read through
+    ``permute(0, 3, 1, 2)`` is image j's channels-last (C, h, w) map, and every row is 32-byte aligned (C >= 8 floats),
+    which the TMA tile kernels of effimvs_warp_corr_agg_f32 need.  At DTU's 1600x1184 that is 26.5 MB per image: about
+    1.3 GB for a 49-image scene, plus 26.5 * K * (n_src + 1) MB for the gathered features of one replay.
+
+    The forward graph starts with the gathers, all driven by one static (K, 1 + n_src) index buffer (reference view,
+    then sources, per batch row): features from the cache, reference images from `imgs`, cameras from `cams`."""
+
+    def __init__(self, model, imgs: torch.Tensor, cams: Dict[str, torch.Tensor], depth_values: torch.Tensor, n_src: int,
+                 views_per_replay: int = 1):
+        if views_per_replay < 1:
+            raise ValueError("views_per_replay must be at least 1, got {}".format(views_per_replay))
+        imgs = imgs.contiguous()
         self.model, self.imgs, self.cams = model, imgs, cams
         self.stages = [k for k in ("stage1", "stage2", "stage3") if k in cams]
-        V = n_src + 1
+        K, V = views_per_replay, n_src + 1
+        self.views_per_replay, self.n_src = K, n_src
         dev = imgs.device
-        self.cache: Dict[int, list] = {}
+        self.encoded_images = set()                  # images whose cache rows hold their features
         self._sel: Dict[tuple, torch.Tensor] = {}
         self.stream = torch.cuda.Stream(dev)
-        self.img_in = imgs[:1].reshape(1, 1, *imgs.shape[1:]).clone()
-        self.ref_in = imgs[:1].clone()
-        self.cam_in = {k: cams[k][:V].unsqueeze(0).clone() for k in self.stages}
-        self.dv = depth_values.reshape(1, -1).clone()
+        self.slot = torch.zeros(1, device=dev, dtype=torch.long)        # the image `encode` reads = the cache row it writes
+        self.idx = torch.zeros(K, V, device=dev, dtype=torch.long)      # the views `forward` reads
+        self.img_in = imgs[:1].clone()
+        self.ref_in = torch.empty(K, *imgs.shape[1:], device=dev, dtype=imgs.dtype)
+        self.cam_in = {k: torch.empty(K, V, *cams[k].shape[1:], device=dev, dtype=cams[k].dtype) for k in self.stages}
+        self.dv = depth_values.reshape(1, -1).repeat(K, 1)
         with torch.no_grad():
             torch.cuda.synchronize(dev)
             with torch.cuda.stream(self.stream):
-                for _ in range(2):                                        # warm-up: cuDNN autotune, lazy init, workspace sizes
-                    enc = [st[0] for st in model.encode(self.img_in)]
-                self.feat_in = [[torch.empty_like(e) for _ in range(V)] for e in enc]
-                for row, e in zip(self.feat_in, enc):
-                    for t in row:
-                        t.copy_(e)
+                enc = [st[0] for st in model.encode(self.img_in.unsqueeze(1))]
+                self.cache = [torch.empty(imgs.shape[0], *e.shape[2:], e.shape[1], device=dev, dtype=e.dtype) for e in enc]
+                self.gathered = [torch.empty(V * K, *c.shape[1:], device=dev, dtype=c.dtype) for c in self.cache]
+                # warm-up (cuDNN autotune, lazy init, workspace sizes) on image 0's features in every view of every row
                 for _ in range(2):
-                    model.forward_from_features(self.feat_in, self.ref_in, self.cam_in, self.dv)
+                    self._encode()
+                for _ in range(2):
+                    self._forward()
             self.stream.synchronize()
             self.g_enc = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.g_enc, stream=self.stream):
-                self.enc_out = [st[0] for st in model.encode(self.img_in)]
+                self._encode()
             self.g_fwd = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.g_fwd, stream=self.stream):
-                out = model.forward_from_features(self.feat_in, self.ref_in, self.cam_in, self.dv)
+                out = self._forward()
             self.out = (out["depth"][-1], out["photometric_confidence"])
 
+    def _encode(self):
+        """image `slot` through the FPN into row `slot` of the cache"""
+        src, dst = _as_words(self.imgs, self.img_in)
+        torch.index_select(src, 0, self.slot, out=dst)
+        for c, e in zip(self.cache, self.model.encode(self.img_in.unsqueeze(1))):
+            dst, src = _as_words(c, e[0].permute(0, 2, 3, 1).contiguous())
+            dst.index_copy_(0, self.slot, src)
+
+    def _forward(self):
+        """the cascade on the K rows of `idx`.  Features are gathered view-major: view v of all K rows is the
+        contiguous channels-last (K, C, h, w) slice v * K .. v * K + K - 1 of the gathered tensor."""
+        K, V = self.idx.shape
+        flat = self.idx.t().reshape(-1)
+        self.feat_in = []
+        for c, g in zip(self.cache, self.gathered):
+            src, dst = _as_words(c, g)
+            torch.index_select(src, 0, flat, out=dst)
+            self.feat_in.append([g[v * K:(v + 1) * K].permute(0, 3, 1, 2) for v in range(V)])
+        src, dst = _as_words(self.imgs, self.ref_in)
+        torch.index_select(src, 0, self.idx[:, 0].contiguous(), out=dst)
+        rows = self.idx.reshape(-1)
+        for k in self.stages:
+            torch.index_select(self.cams[k], 0, rows, out=self.cam_in[k].view(K * V, *self.cams[k].shape[1:]))
+        return self.model.forward_from_features(self.feat_in, self.ref_in, self.cam_in, self.dv)
+
     def _index(self, idx):
-        """device index tensor of a view list, built once: a host list -> device copy is a stream synchronisation, and one per
-        view serialises the host's enqueue work with the previous view's graph"""
-        key = tuple(idx)
+        """device tensor of an index list, built once per distinct list: a host list -> device copy is a stream
+        synchronisation, and one per replay would serialise the host's enqueue work with the previous replay"""
+        key = tuple(map(tuple, idx)) if idx and isinstance(idx[0], (list, tuple)) else tuple(idx)
         if key not in self._sel:
-            self._sel[key] = torch.as_tensor(list(idx), device=self.imgs.device)
+            self._sel[key] = torch.as_tensor(idx, device=self.imgs.device, dtype=torch.long)
         return self._sel[key]
 
-    @torch.no_grad()
-    def encoded(self, j: int):
-        if j not in self.cache:
-            self.img_in.copy_(self.imgs[j].reshape(self.img_in.shape))
-            self.g_enc.replay()
-            self.cache[j] = [e.clone() for e in self.enc_out]
-        return self.cache[j]
+    def clear_cache(self):
+        """forget which images are encoded: the next replays encode them again"""
+        self.encoded_images.clear()
 
     @torch.no_grad()
-    def infer(self, i: int, srcs: Sequence[int]):
-        idx = [i] + list(srcs)
-        if len(idx) != len(self.feat_in[0]):
-            raise ValueError("GraphedViewRunner was captured for {} source views, got {}".format(len(self.feat_in[0]) - 1, len(srcs)))
+    def infer_batch(self, items: Sequence):
+        """items: up to K (reference view, source views) pairs -> [(depth (H,W), conf (hc,wc))] in the same order.
+        A short batch is padded with its last view; the padded rows' outputs are dropped."""
+        if not 0 < len(items) <= self.views_per_replay:
+            raise ValueError("GraphedViewRunner takes 1 to {} views per replay, got {}".format(self.views_per_replay, len(items)))
+        for _, srcs in items:
+            if len(srcs) != self.n_src:
+                raise ValueError("GraphedViewRunner was captured for {} source views, got {}".format(self.n_src, len(srcs)))
+        (rows, n), = view_groups([[i] + list(srcs) for i, srcs in items], self.views_per_replay)
         with torch.cuda.stream(self.stream):
-            for v, j in enumerate(idx):
-                for s, e in enumerate(self.encoded(j)):
-                    self.feat_in[s][v].copy_(e)
-            self.ref_in.copy_(self.imgs[i:i + 1])
-            sel = self._index(idx)
-            for k in self.stages:
-                self.cam_in[k].copy_(self.cams[k].index_select(0, sel).unsqueeze(0))
+            for j in (j for row in rows[:n] for j in row):
+                if j not in self.encoded_images:
+                    self.slot.copy_(self._index([j]))
+                    self.g_enc.replay()
+                    self.encoded_images.add(j)
+            self.idx.copy_(self._index(rows))
             self.g_fwd.replay()
-            depth, conf = self.out[0][0].clone(), self.out[1][0].clone()
+            depth, conf = self.out[0][:n].clone(), self.out[1][:n].clone()     # before the next replay overwrites them
         torch.cuda.current_stream().wait_stream(self.stream)
-        return depth, conf
+        return [(depth[b], conf[b]) for b in range(n)]
 
 
 def cuda_scene_callables(model, imgs: torch.Tensor, cams: Dict[str, torch.Tensor], depth_values: torch.Tensor,
                          dist_base: float, rel_diff_base: float, thres_view: int, prob_threshold: float,
-                         feature_cache: bool = False, graphed_src_views: int = 0):
+                         feature_cache: bool = False, graphed_src_views: int = 0, views_per_replay: int = 1):
     """infer / fuse callables for `run_scene` on the CUDA path.
     imgs (Nv,3,H,W) on the device; cams {"stage1".."stage4": (Nv,2,4,4)}; depth_values (Dv).
     feature_cache: encode every image once per rank and reuse its feature pyramid for each reference view
     that lists it as a source (section 8(f) row 1; eval-mode results are those of re-encoding it).
     graphed_src_views > 0: run encode / cascade as CUDA graphs captured for that many source views (implies the
-    feature cache)."""
+    feature cache); then infer.batch([(ref_view, src_views), ...]) runs up to views_per_replay views per replay of the
+    cascade, and run_scene groups the views accordingly.  views_per_replay > 1 needs the graphs."""
     from . import fusion
+    if views_per_replay != 1 and graphed_src_views <= 0:
+        raise ValueError("views_per_replay = {} needs graphed_src_views > 0 (views are batched inside the CUDA graph)".format(views_per_replay))
     cache: Dict[int, list] = {}
-    runner = GraphedViewRunner(model, imgs, cams, depth_values, graphed_src_views) if graphed_src_views > 0 else None
+    runner = GraphedViewRunner(model, imgs, cams, depth_values, graphed_src_views, views_per_replay) if graphed_src_views > 0 else None
 
     def encoded(j):
         if j not in cache:
@@ -217,7 +297,7 @@ def cuda_scene_callables(model, imgs: torch.Tensor, cams: Dict[str, torch.Tensor
 
     def infer(i, srcs):
         if runner is not None:
-            return runner.infer(i, srcs)
+            return runner.infer_batch([(i, srcs)])[0]
         idx = [i] + list(srcs)
         stage_cams = {k: v[idx].unsqueeze(0) for k, v in cams.items() if k != "stage4"}
         if feature_cache:
@@ -228,11 +308,15 @@ def cuda_scene_callables(model, imgs: torch.Tensor, cams: Dict[str, torch.Tensor
             out = model(imgs[idx].unsqueeze(0), stage_cams, depth_values.unsqueeze(0))
         return out["depth"][-1][0], out["photometric_confidence"][0]
 
+    if runner is not None:
+        infer.batch = runner.infer_batch
+        infer.views_per_batch = views_per_replay
+
     def clear_cache():
         """forget the encoded feature pyramids (a new scene, or a benchmark pass that must encode again)"""
         cache.clear()
         if runner is not None:
-            runner.cache.clear()
+            runner.clear_cache()
     infer.clear_cache = clear_cache
 
     sel_cache: Dict[tuple, torch.Tensor] = {}
