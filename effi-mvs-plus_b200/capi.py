@@ -86,6 +86,8 @@ SIGNATURES = {
     "effimvs_gru_init_ctx_f32": (_i, [_p, C.c_longlong, _i, _i, _p, _p, _p, _p, _p]),
     "effimvs_dtu_filter_f32": (_i, [_p, _p, _p, _p, C.POINTER(C.c_double), C.POINTER(C.c_float), _i, _i, _i, _f, _f, _i, _i, _i,
                                     _p, _p, _p, _p, _p, _p, _p]),
+    "effimvs_dtu_filter_views_f32": (_i, [_p, _i, _p, _p, _p, _i, _p, _p, C.POINTER(C.c_double), C.POINTER(C.c_float), _i, _i, _i,
+                                          _f, _f, _i, _i, _i, _p, _p, _p, _p, _p]),
     "effimvs_images_u8_to_f32": (_i, [_p, C.c_longlong, _p, _p]),
     "effimvs_fusion_invert_cameras_f32": (_i, [_p, _p, _i, _i, _p, _p]),
     "effimvs_fusion_reproject_f32": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p]),

@@ -59,18 +59,16 @@ __device__ __forceinline__ float remap_bilinear(const float* __restrict__ img, i
 // mats: [Kinv_ref 9][K_ref 9][Einv_ref 16] then per source view [E_src @ inv(E_ref) 16][K_src 9][Kinv_src 9][E_ref @ inv(E_src) 16]
 constexpr int REF_FLOATS = 34, SRC_FLOATS = 50;
 
-__global__ void __launch_bounds__(128)
-dtu_filter_kernel(const float* __restrict__ ref_depth, const float* __restrict__ srcs_depth, const float* __restrict__ conf,
-                  const float* __restrict__ mats, const __grid_constant__ Ladder lad, int K, int S, int E, float conf_thres,
-                  float conf_keep, int v, int h, int w, uint8_t* __restrict__ final_mask, uint8_t* __restrict__ geo_mask,
-                  float* __restrict__ depth_avg, float* __restrict__ points, uint8_t* __restrict__ masks_out,
-                  float* __restrict__ reproj_depth_out) {
-    extern __shared__ float sm[];   // REF_FLOATS + v * SRC_FLOATS
-    for (int i = threadIdx.x; i < REF_FLOATS + v * SRC_FLOATS; i += blockDim.x) sm[i] = mats[i];
-    __syncthreads();
+// One reference pixel of the filter.  `src_of(s)` is source view s's (h,w) depth map; the output pointers are the
+// view's own (h,w) / (3,h,w) planes; geo_mask, masks_out and reproj_depth_out may be null.
+template <class SrcOf>
+__device__ __forceinline__ void dtu_filter_pixel(int pix, const float* __restrict__ sm, const float* __restrict__ ref_depth,
+                                                 SrcOf src_of, const float* __restrict__ conf, const Ladder& lad, int K, int S,
+                                                 int E, float conf_thres, float conf_keep, int v, int h, int w,
+                                                 uint8_t* __restrict__ final_mask, uint8_t* __restrict__ geo_mask,
+                                                 float* __restrict__ depth_avg, float* __restrict__ points,
+                                                 uint8_t* __restrict__ masks_out, float* __restrict__ reproj_depth_out) {
     const int hw = h * w;
-    const int pix = blockIdx.x * blockDim.x + threadIdx.x;
-    if (pix >= hw) return;
     const int yi = pix / w, xi = pix - yi * w;
     const double xd = (double)xi, yd = (double)yi;
     const float dref = __ldg(ref_depth + pix);
@@ -89,7 +87,7 @@ dtu_filter_kernel(const float* __restrict__ ref_depth, const float* __restrict__
         mat4d(R1, pr, ps);
         mat3d(K_src, ps[0], ps[1], ps[2], ks);
         const double u = __ddiv_rn(ks[0], ks[2]), t = __ddiv_rn(ks[1], ks[2]);
-        const float sampled = remap_bilinear(srcs_depth + (size_t)s * hw, h, w, (float)u, (float)t);
+        const float sampled = remap_bilinear(src_of(s), h, w, (float)u, (float)t);
         const double sd = (double)sampled;
         double q[3], back[3], kb[3];
         mat3d(Kinv_src, __dmul_rn(u, sd), __dmul_rn(t, sd), sd, q);
@@ -139,6 +137,61 @@ dtu_filter_kernel(const float* __restrict__ ref_depth, const float* __restrict__
     points[(size_t)2 * hw + pix] = (float)pw[2];
 }
 
+__global__ void __launch_bounds__(128)
+dtu_filter_kernel(const float* __restrict__ ref_depth, const float* __restrict__ srcs_depth, const float* __restrict__ conf,
+                  const float* __restrict__ mats, const __grid_constant__ Ladder lad, int K, int S, int E, float conf_thres,
+                  float conf_keep, int v, int h, int w, uint8_t* __restrict__ final_mask, uint8_t* __restrict__ geo_mask,
+                  float* __restrict__ depth_avg, float* __restrict__ points, uint8_t* __restrict__ masks_out,
+                  float* __restrict__ reproj_depth_out) {
+    extern __shared__ float sm[];   // REF_FLOATS + v * SRC_FLOATS
+    for (int i = threadIdx.x; i < REF_FLOATS + v * SRC_FLOATS; i += blockDim.x) sm[i] = mats[i];
+    __syncthreads();
+    const int hw = h * w;
+    const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pix >= hw) return;
+    dtu_filter_pixel(pix, sm, ref_depth, [&](int s) { return srcs_depth + (size_t)s * hw; }, conf, lad, K, S, E, conf_thres,
+                     conf_keep, v, h, w, final_mask, geo_mask, depth_avg, points, masks_out, reproj_depth_out);
+}
+
+// Several reference views in one launch: grid (pixel tiles of 128, n views).  Block y filters reference view y, whose
+// depth map and source maps are rows ref_idx[y] and src_idx[y][0 .. src_count[y]) of the one (N,h,w) depth stack, read
+// in place; its camera pack is row y of `mats` (REF_FLOATS + vmax * SRC_FLOATS floats, the single-view layout padded to
+// vmax sources).  Every view's results are those of dtu_filter_kernel on that view alone.
+__global__ void __launch_bounds__(128)
+dtu_filter_views_kernel(const float* __restrict__ depths, const int* __restrict__ ref_idx, const int* __restrict__ src_idx,
+                        const int* __restrict__ src_count, int vmax, const float* __restrict__ mats,
+                        const float* __restrict__ conf, const __grid_constant__ Ladder lad, int K, int S, int E,
+                        float conf_thres, float conf_keep, int h, int w, uint8_t* __restrict__ final_mask,
+                        uint8_t* __restrict__ geo_mask, float* __restrict__ depth_avg, float* __restrict__ points) {
+    extern __shared__ float sm[];   // REF_FLOATS + vmax * SRC_FLOATS floats, then vmax source rows (int)
+    int* rows = reinterpret_cast<int*>(sm + REF_FLOATS + vmax * SRC_FLOATS);
+    const int view = blockIdx.y;
+    const int v = src_count[view];
+    const float* pack = mats + (size_t)view * (REF_FLOATS + vmax * SRC_FLOATS);
+    for (int i = threadIdx.x; i < REF_FLOATS + v * SRC_FLOATS; i += blockDim.x) sm[i] = pack[i];
+    for (int i = threadIdx.x; i < v; i += blockDim.x) rows[i] = src_idx[(size_t)view * vmax + i];
+    __syncthreads();
+    const int hw = h * w;
+    const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pix >= hw) return;
+    const size_t plane = (size_t)view * hw;
+    dtu_filter_pixel(pix, sm, depths + (size_t)ref_idx[view] * hw, [&](int s) { return depths + (size_t)rows[s] * hw; },
+                     conf + plane, lad, K, S, E, conf_thres, conf_keep, v, h, w, final_mask + plane,
+                     geo_mask ? geo_mask + plane : nullptr, depth_avg + plane, points + 3 * plane, nullptr, nullptr);
+}
+
+// the rung thresholds as the kernels' parameter block; fails unless both ladders are non-decreasing
+int make_ladder(const double* thr_dist_host, const float* thr_diff_host, int n_rungs, Ladder* lad) {
+    for (int k = 0; k < MAX_RUNGS; ++k) {
+        lad->dist[k] = k < n_rungs ? thr_dist_host[k] : 0.0;
+        lad->diff[k] = k < n_rungs ? thr_diff_host[k] : 0.0f;
+        if (k > 0 && k < n_rungs)
+            EFFI_REQUIRE(lad->dist[k] >= lad->dist[k - 1] && lad->diff[k] >= lad->diff[k - 1], EFFIMVS_EUNSUPPORTED,
+                         "dtu_filter: the threshold ladder must be non-decreasing");
+    }
+    return EFFIMVS_OK;
+}
+
 }  // namespace
 }  // namespace effimvs
 
@@ -154,17 +207,32 @@ extern "C" int effimvs_dtu_filter_f32(const float* ref_depth, const float* srcs_
     EFFI_REQUIRE(v >= 1 && v <= 31 && h > 1 && w > 1, EFFIMVS_EINVAL, "dtu_filter: bad sizes (v in [1,31])");
     EFFI_REQUIRE(n_rungs >= 1 && n_rungs <= MAX_RUNGS && first_rung >= 0, EFFIMVS_EINVAL, "dtu_filter: n_rungs=%d outside [1,%d]", n_rungs, MAX_RUNGS);
     Ladder lad;
-    for (int k = 0; k < MAX_RUNGS; ++k) {
-        lad.dist[k] = k < n_rungs ? thr_dist_host[k] : 0.0;
-        lad.diff[k] = k < n_rungs ? thr_diff_host[k] : 0.0f;
-        if (k > 0 && k < n_rungs)
-            EFFI_REQUIRE(lad.dist[k] >= lad.dist[k - 1] && lad.diff[k] >= lad.diff[k - 1], EFFIMVS_EUNSUPPORTED,
-                         "dtu_filter: the threshold ladder must be non-decreasing");
-    }
+    if (const int rc = make_ladder(thr_dist_host, thr_diff_host, n_rungs, &lad)) return rc;
     dim3 block(128), grid(ceil_div(h * w, 128));
     const size_t smem = (size_t)(REF_FLOATS + v * SRC_FLOATS) * sizeof(float);
     dtu_filter_kernel<<<grid, block, smem, (cudaStream_t)stream>>>(ref_depth, srcs_depth, conf, mats, lad, n_rungs, first_rung, full_count,
                                                                   conf_thres, conf_keep, v, h, w, final_mask, geo_mask, depth_avg, points,
                                                                   masks_out, reproj_depth_out);
     return check_launch("dtu_filter_kernel");
+}
+
+extern "C" int effimvs_dtu_filter_views_f32(const float* depths, int n_depths, const int* ref_idx, const int* src_idx,
+                                            const int* src_count, int vmax, const float* mats, const float* conf,
+                                            const double* thr_dist_host, const float* thr_diff_host, int n_rungs, int first_rung,
+                                            int full_count, float conf_thres, float conf_keep, int n, int h, int w,
+                                            uint8_t* final_mask, uint8_t* geo_mask, float* depth_avg, float* points, void* stream) {
+    EFFI_REQUIRE(depths && ref_idx && src_idx && src_count && mats && conf && thr_dist_host && thr_diff_host && final_mask &&
+                 depth_avg && points, EFFIMVS_EINVAL, "dtu_filter_views: null pointer");
+    EFFI_REQUIRE(n_depths >= 1 && vmax >= 1 && vmax <= 31 && n >= 1 && n <= 65535 && h > 1 && w > 1 &&
+                 (long long)h * w <= 0x7fffffffLL - 127, EFFIMVS_EINVAL,
+                 "dtu_filter_views: bad sizes (N=%d, vmax=%d in [1,31], n=%d in [1,65535], h=%d, w=%d)", n_depths, vmax, n, h, w);
+    EFFI_REQUIRE(n_rungs >= 1 && n_rungs <= MAX_RUNGS && first_rung >= 0, EFFIMVS_EINVAL, "dtu_filter_views: n_rungs=%d outside [1,%d]", n_rungs, MAX_RUNGS);
+    Ladder lad;
+    if (const int rc = make_ladder(thr_dist_host, thr_diff_host, n_rungs, &lad)) return rc;
+    dim3 block(128), grid(ceil_div(h * w, 128), n);
+    const size_t smem = (size_t)(REF_FLOATS + vmax * SRC_FLOATS) * sizeof(float) + (size_t)vmax * sizeof(int);
+    dtu_filter_views_kernel<<<grid, block, smem, (cudaStream_t)stream>>>(depths, ref_idx, src_idx, src_count, vmax, mats, conf, lad,
+                                                                        n_rungs, first_rung, full_count, conf_thres, conf_keep, h, w,
+                                                                        final_mask, geo_mask, depth_avg, points);
+    return check_launch("dtu_filter_views_kernel");
 }

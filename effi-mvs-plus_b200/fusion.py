@@ -70,6 +70,15 @@ def dtu_camera_pack(K_ref, E_ref, Ks_src, Es_src):
     return torch.from_numpy(np.concatenate(parts).astype(np.float32))
 
 
+def dtu_ladder(first_rung: int, end_rung: int, dist_base: float, diff_base: float):
+    """the rung thresholds of check_geometric_consistency (test_dtu_dypcd.py:226-228): i * dist_base as float64 and
+    log10(max(i, 1.05)) * diff_base rounded to float32, i = first_rung .. end_rung - 1"""
+    import math
+    import numpy as np
+    rungs = range(first_rung, end_rung)
+    return [i * dist_base for i in rungs], [float(np.float32(math.log(max(i, 1.05), 10) * diff_base)) for i in rungs]
+
+
 def dtu_filter_view(ref_depth, confidence, srcs_depth, K_ref, E_ref, Ks_src, Es_src, conf_thres: float = 0.5,
                     want_masks: bool = False, first_rung: int = DTU_FIRST_RUNG, end_rung: int = DTU_END_RUNG,
                     dist_base: float = DTU_DIST_BASE, diff_base: float = DTU_DIFF_BASE):
@@ -78,15 +87,11 @@ def dtu_filter_view(ref_depth, confidence, srcs_depth, K_ref, E_ref, Ks_src, Es_
     ref_depth (h,w), srcs_depth (v,h,w) CUDA fp32; confidence (hc,wc) CUDA fp32, resized to (h,w) bilinearly with
     half-pixel centres like cv2.resize (:258) when the sizes differ; cameras as host arrays (3x3 / 4x4).
     -> dict(final, geo (h,w) bool, depth_avg (h,w), points (3,h,w)[, masks (v,K,h,w) bool, reproj_depth (v,h,w)])."""
-    import math
-    import numpy as np
     h, w = ref_depth.shape[-2:]
     if tuple(confidence.shape[-2:]) != (h, w):
         confidence = torch.nn.functional.interpolate(confidence.reshape(1, 1, *confidence.shape[-2:]), size=(h, w), mode="bilinear",
                                                      align_corners=False).reshape(h, w)
-    rungs = range(first_rung, end_rung)
-    thr_dist = [i * dist_base for i in rungs]
-    thr_diff = [float(np.float32(math.log(max(i, 1.05), 10) * diff_base)) for i in rungs]
+    thr_dist, thr_diff = dtu_ladder(first_rung, end_rung, dist_base, diff_base)
     mats = dtu_camera_pack(K_ref, E_ref, Ks_src, Es_src).to(ref_depth.device)
     final, geo, avg, pts, masks, rep = ops.dtu_filter(ref_depth.reshape(h, w), srcs_depth.reshape(-1, h, w), confidence.reshape(h, w), mats,
                                                       thr_dist, thr_diff, first_rung, end_rung, float(conf_thres), 0.75, bool(want_masks))
@@ -94,3 +99,112 @@ def dtu_filter_view(ref_depth, confidence, srcs_depth, K_ref, E_ref, Ks_src, Es_
     if want_masks:
         out["masks"], out["reproj_depth"] = masks.bool(), rep
     return out
+
+
+# ---- the same filter for a whole scene: all of a rank's reference views in one launch -----------------------------
+DTU_MAX_SOURCES = 31          # the kernel's histogram limit
+
+
+class DtuSceneCameras:
+    """The DTU filter's camera packs of every view of a scene, built once on the host (see dtu_scene_cameras).
+
+    mats (N, 34 + 50 vmax) float32: row i is dtu_camera_pack of view i and its sources, zero padded to vmax sources;
+    src (N, vmax) int32: the sources of view i, zero padded; count (N,) int32: their number."""
+
+    def __init__(self, mats: torch.Tensor, src: torch.Tensor, count: torch.Tensor):
+        self.mats, self.src, self.count = mats, src, count
+        self.n_views, self.vmax = src.shape
+        self._rows = {}
+
+    def rows(self, views, device, stack_rows=None):
+        """the device arrays of effimvs_dtu_filter_views_f32 for reference views `views` (in that order):
+        (ref_idx (n,), src_idx (n,vmax), src_count (n,) int32, mats (n, 34 + 50 vmax) float32).  Indices are scene view
+        numbers, or stack_rows[view] where the depth stack holds the scene's maps in another order.  Built and uploaded in
+        one host -> device copy the first time a list is asked for, then cached: a host -> device copy synchronises the
+        host with the stream and cannot be captured in a CUDA graph, so the first call for a list comes before a capture."""
+        views = [int(i) for i in views]
+        key = (tuple(views), str(device), None if stack_rows is None else tuple(sorted(stack_rows.items())))
+        if key not in self._rows:
+            for i in views:
+                if not 0 <= i < self.n_views:
+                    raise ValueError("view {} is outside the scene's {} views".format(i, self.n_views))
+            n, R = len(views), self.mats.shape[1]
+            sel = torch.as_tensor(views, dtype=torch.long)
+            ref, src = sel.to(torch.int32), self.src[sel]
+            if stack_rows is not None:
+                ref = torch.as_tensor([stack_rows[i] for i in views], dtype=torch.int32)
+                for b, i in enumerate(views):
+                    c = int(self.count[i])
+                    src[b, :c] = torch.as_tensor([stack_rows[int(j)] for j in self.src[i, :c]], dtype=torch.int32)
+            host = torch.cat([ref, src.reshape(-1), self.count[sel], self.mats[sel].view(torch.int32).reshape(-1)])
+            dev = host.to(device)
+            a, b, c = n, n + n * self.vmax, 2 * n + n * self.vmax
+            self._rows[key] = (dev[:a], dev[a:b].view(n, self.vmax), dev[b:c], dev[c:].view(torch.float32).view(n, R))
+        return self._rows[key]
+
+
+def dtu_scene_cameras(K, E, fuse_pairs) -> DtuSceneCameras:
+    """Camera packs of every view of a scene for the batched DTU filter.  K (N,3,3), E (N,4,4) host arrays (float32, as
+    upstream reads them from the cam files); fuse_pairs[i]: the 1 .. 31 source views of view i.  Row i is
+    dtu_camera_pack(K[i], E[i], K[fuse_pairs[i]], E[fuse_pairs[i]]) bit for bit: the same NumPy float32 calls."""
+    import numpy as np
+    K = np.asarray(K.cpu() if torch.is_tensor(K) else K, dtype=np.float32)
+    E = np.asarray(E.cpu() if torch.is_tensor(E) else E, dtype=np.float32)
+    N = K.shape[0]
+    if K.shape != (N, 3, 3) or E.shape != (N, 4, 4):
+        raise ValueError("K (N,3,3) and E (N,4,4) of the same N, got {} and {}".format(K.shape, E.shape))
+    if len(fuse_pairs) != N:
+        raise ValueError("{} source lists for {} views".format(len(fuse_pairs), N))
+    pairs = [[int(j) for j in p] for p in fuse_pairs]
+    for i, p in enumerate(pairs):
+        if not 1 <= len(p) <= DTU_MAX_SOURCES:
+            raise ValueError("view {} has {} source views; the DTU filter takes 1 to {}".format(i, len(p), DTU_MAX_SOURCES))
+        if any(not 0 <= j < N for j in p):
+            raise ValueError("view {}: source views {} are outside the scene's {} views".format(i, p, N))
+    vmax = max(len(p) for p in pairs)
+    mats = torch.zeros(N, 34 + 50 * vmax, dtype=torch.float32)
+    src = torch.zeros(N, vmax, dtype=torch.int32)
+    for i, p in enumerate(pairs):
+        row = dtu_camera_pack(K[i], E[i], [K[j] for j in p], [E[j] for j in p])
+        mats[i, :row.numel()] = row
+        src[i, :len(p)] = torch.as_tensor(p, dtype=torch.int32)
+    return DtuSceneCameras(mats, src, torch.as_tensor([len(p) for p in pairs], dtype=torch.int32))
+
+
+def dtu_filter_views(depth_stack, views, confs, table: DtuSceneCameras, conf_thres: float = 0.5, stack_rows=None,
+                     first_rung: int = DTU_FIRST_RUNG, end_rung: int = DTU_END_RUNG, dist_base: float = DTU_DIST_BASE,
+                     diff_base: float = DTU_DIFF_BASE):
+    """Upstream's DTU ``filter_depth`` (test_dtu_dypcd.py:236-337) for the reference views `views` in ONE launch.
+
+    depth_stack (N,h,w) CUDA fp32 holds the depth map of every view of the scene (the scene runner's all-gathered maps);
+    each view's reference and source maps are read from it in place.  stack_rows: {view: row of depth_stack} when the
+    stack is not in scene order (default: view i is row i, and N is the scene's view count).  confs (n,hc,wc) CUDA fp32,
+    resized to (h,w) as dtu_filter_view does; table from dtu_scene_cameras.  Makes no host synchronisation once the
+    table's rows for `views` are on the device (table.rows), so it can be captured in a CUDA graph.
+    -> dict(final, geo (n,h,w) bool, depth_avg (n,h,w), points (n,3,h,w)); view views[b]'s results are bit-identical to
+    dtu_filter_view on that view alone."""
+    views = [int(i) for i in views]
+    if not views:
+        raise ValueError("no reference view to filter")
+    if any(not 0 <= i < table.n_views for i in views):
+        raise ValueError("views {} are not all inside the scene's {} views".format(views, table.n_views))
+    if depth_stack.dim() != 3:
+        raise ValueError("depth_stack must be (N,h,w), got {}".format(tuple(depth_stack.shape)))
+    N, h, w = depth_stack.shape
+    if stack_rows is None and N != table.n_views:
+        raise ValueError("the depth stack holds {} maps, the camera table {} views".format(N, table.n_views))
+    if stack_rows is not None:
+        need = set(views) | {int(j) for i in views for j in table.src[i, :int(table.count[i])]}
+        if any(i not in stack_rows or not 0 <= stack_rows[i] < N for i in need):
+            raise ValueError("views {} are not all rows of the {}-map depth stack".format(sorted(need), N))
+    n = len(views)
+    if confs.dim() != 3 or confs.shape[0] != n:
+        raise ValueError("confs must be (n,hc,wc) for n = {} views, got {}".format(n, tuple(confs.shape)))
+    if tuple(confs.shape[-2:]) != (h, w):
+        confs = torch.nn.functional.interpolate(confs.reshape(n, 1, *confs.shape[-2:]), size=(h, w), mode="bilinear",
+                                                align_corners=False).reshape(n, h, w)
+    thr_dist, thr_diff = dtu_ladder(first_rung, end_rung, dist_base, diff_base)
+    ref, src, count, mats = table.rows(views, depth_stack.device, stack_rows)
+    final, geo, avg, pts = ops.dtu_filter_views(depth_stack, ref, src, count, mats, confs, thr_dist, thr_diff, first_rung,
+                                                end_rung, float(conf_thres), 0.75)
+    return {"final": final.bool(), "geo": geo.bool(), "depth_avg": avg, "points": pts}

@@ -1066,3 +1066,48 @@ def _(ref_depth, srcs_depth, conf, mats, thr_dist, thr_diff, first_rung, full_co
     return (ref_depth.new_empty(h, w, dtype=u8), ref_depth.new_empty(h, w, dtype=u8), ref_depth.new_empty(h, w),
             ref_depth.new_empty(3, h, w), ref_depth.new_empty((v, K, h, w) if want_masks else (0,), dtype=u8),
             ref_depth.new_empty((v, h, w) if want_masks else (0,)))
+
+
+def _dev_i32(t: Tensor, name: str) -> Tensor:
+    if not t.is_cuda:
+        raise RuntimeError("effimvs::{} got a CPU tensor; the hot path is CUDA-only (no fallback)".format(name))
+    return (t if t.dtype == torch.int32 else t.int()).contiguous()
+
+
+@torch.library.custom_op("effimvs::dtu_filter_views", mutates_args=())
+@_on_tensor_device
+def dtu_filter_views(depths: Tensor, ref_idx: Tensor, src_idx: Tensor, src_count: Tensor, mats: Tensor, conf: Tensor,
+                     thr_dist: List[float], thr_diff: List[float], first_rung: int, full_count: int, conf_thres: float,
+                     conf_keep: float) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """n reference views of one scene in one launch.  depths (N,h,w); ref_idx (n), src_idx (n,vmax), src_count (n) int32
+    rows of `depths` (NOT checked on the device: the caller validates its host lists); mats (n, 34 + 50 vmax);
+    conf (n,h,w).  -> final (n,h,w) u8, geo (n,h,w) u8, depth_avg (n,h,w), points (n,3,h,w)."""
+    import ctypes
+    depths, mats, conf = _dev(depths, "dtu_filter_views"), _dev(mats, "dtu_filter_views"), _dev(conf, "dtu_filter_views")
+    ref_idx, src_idx, src_count = (_dev_i32(ref_idx, "dtu_filter_views"), _dev_i32(src_idx, "dtu_filter_views"),
+                                   _dev_i32(src_count, "dtu_filter_views"))
+    N, h, w = depths.shape
+    n, vmax = src_idx.shape
+    K = len(thr_dist)
+    dev = depths.device
+    final = torch.empty(n, h, w, device=dev, dtype=torch.uint8)
+    geo = torch.empty(n, h, w, device=dev, dtype=torch.uint8)
+    avg = torch.empty(n, h, w, device=dev, dtype=torch.float32)
+    pts = torch.empty(n, 3, h, w, device=dev, dtype=torch.float32)
+    td = (ctypes.c_double * K)(*thr_dist)
+    tf = (ctypes.c_float * K)(*thr_diff)
+    _count(1)
+    capi.check(_lib.effimvs_dtu_filter_views_f32(depths.data_ptr(), N, ref_idx.data_ptr(), src_idx.data_ptr(), src_count.data_ptr(),
+                                                 vmax, mats.data_ptr(), conf.data_ptr(), td, tf, K, first_rung, full_count,
+                                                 conf_thres, conf_keep, n, h, w, final.data_ptr(), geo.data_ptr(), avg.data_ptr(),
+                                                 pts.data_ptr(), _stream()))
+    return final, geo, avg, pts
+
+
+@dtu_filter_views.register_fake
+def _(depths, ref_idx, src_idx, src_count, mats, conf, thr_dist, thr_diff, first_rung, full_count, conf_thres, conf_keep):
+    _, h, w = depths.shape
+    n = src_idx.shape[0]
+    u8 = torch.uint8
+    return (depths.new_empty(n, h, w, dtype=u8), depths.new_empty(n, h, w, dtype=u8), depths.new_empty(n, h, w),
+            depths.new_empty(n, 3, h, w))

@@ -100,6 +100,9 @@ def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Seq
     views whose depth maps the consistency filter of view i reads (upstream: 4 and up to 10).
     When infer has `batch` (infer.batch([(ref_view, src_views), ...]) -> [(depth, conf), ...]), the rank's views go to
     it in view order, in groups of at most views_per_batch (default: infer.views_per_batch, else 1).
+    When fuse has `batch`, it is called once for all of the rank's views instead of fuse per view:
+    fuse.batch(views in order, all depth maps (n_views,h,w), confs (n,hc,wc), fuse_pairs) -> dict with 'final'
+    (n,1,h,w) bool and 'points' (n,3,h,w).
     Returns {ref_view: (points (k,3), depth (h,w))} for the views this rank owns."""
     fuse_pairs = pairs if fuse_pairs is None else fuse_pairs
     mine = shard_views(n_views, rank, world, sharding)
@@ -130,16 +133,24 @@ def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Seq
     if ev:
         ev[1].record()
     out = {}
-    flat = [j for i in mine for j in fuse_pairs[i]]
-    flat_dev = torch.as_tensor(flat, device=all_depths.device, dtype=torch.long) if flat else None      # ONE host -> device copy
-    at = 0
-    for i in mine:
-        src = list(fuse_pairs[i])
-        sel = flat_dev[at:at + len(src)]
-        at += len(src)
-        res = fuse(i, depths[i].reshape(1, 1, h, w), confs[i].unsqueeze(0), src, all_depths.index_select(0, sel).reshape(1, len(src), 1, h, w))
-        m = res["final"][0, 0]
-        out[i] = (res["points"][0][:, m].t().contiguous(), depths[i])
+    fuse_batch = getattr(fuse, "batch", None)
+    if fuse_batch is not None:
+        if mine:
+            res = fuse_batch(mine, all_depths, torch.stack([confs[i] for i in mine]), fuse_pairs)
+            for b, i in enumerate(mine):
+                m = res["final"][b, 0]
+                out[i] = (res["points"][b][:, m].t().contiguous(), depths[i])
+    else:
+        flat = [j for i in mine for j in fuse_pairs[i]]
+        flat_dev = torch.as_tensor(flat, device=all_depths.device, dtype=torch.long) if flat else None      # ONE host -> device copy
+        at = 0
+        for i in mine:
+            src = list(fuse_pairs[i])
+            sel = flat_dev[at:at + len(src)]
+            at += len(src)
+            res = fuse(i, depths[i].reshape(1, 1, h, w), confs[i].unsqueeze(0), src, all_depths.index_select(0, sel).reshape(1, len(src), 1, h, w))
+            m = res["final"][0, 0]
+            out[i] = (res["points"][0][:, m].t().contiguous(), depths[i])
     if ev:
         ev[2].record()
         torch.cuda.synchronize()
@@ -329,3 +340,39 @@ def cuda_scene_callables(model, imgs: torch.Tensor, cams: Dict[str, torch.Tensor
         return fusion.filter_view(ref_depth, conf, src_depths, full[i].unsqueeze(0), full.index_select(0, sel_cache[key]).unsqueeze(0),
                                   dist_base, rel_diff_base, thres_view, prob_threshold, torch_inverse=False)
     return infer, fuse
+
+
+def cuda_dtu_fuse(cams_stage4: torch.Tensor, fuse_pairs: Sequence[Sequence[int]], conf_thres: float = 0.5):
+    """A `fuse` callable for run_scene with upstream's DTU filter (test_dtu_dypcd.py:236-337, fusion.dtu_filter_view)
+    instead of the dynamic filter of cuda_scene_callables; use it with that function's `infer`.
+
+    cams_stage4 (Nv,2,4,4): E = [:, 0], K = [:, 1, :3, :3], taken to the host as float32 as upstream reads them from the
+    cam files; fuse_pairs[i]: the 1 .. 31 source views of view i.  The camera table of the whole scene is built once.
+    fuse.batch(views, all_depths, confs, fuse_pairs) filters all of a rank's views in one launch, reading every depth
+    map in place from the all-gathered (Nv,h,w) tensor; the per-view call runs the same kernel with n = 1 on a stack
+    of its own maps.  Both take the scene's fuse_pairs and raise ValueError for any other source list."""
+    from . import fusion
+    cams = cams_stage4.detach().to("cpu", torch.float32)
+    pairs = [[int(j) for j in p] for p in fuse_pairs]
+    table = fusion.dtu_scene_cameras(cams[:, 1, :3, :3].numpy(), cams[:, 0].numpy(), pairs)
+
+    def same_sources(i, srcs):
+        if [int(j) for j in srcs] != pairs[i]:
+            raise ValueError("view {}: source views {} differ from the {} this fuse was built for".format(i, list(srcs), pairs[i]))
+
+    def fuse(i, ref_depth, conf, srcs, src_depths):
+        same_sources(i, srcs)
+        h, w = ref_depth.shape[-2:]
+        stack = torch.cat([ref_depth.reshape(1, h, w), src_depths.reshape(-1, h, w)])
+        rows = {j: 1 + b for b, j in reversed(list(enumerate(pairs[i])))}
+        rows[i] = 0
+        res = fusion.dtu_filter_views(stack, [i], conf.reshape(1, *conf.shape[-2:]), table, conf_thres, stack_rows=rows)
+        return {"final": res["final"].unsqueeze(1), "points": res["points"]}
+
+    def batch(views, all_depths, confs, fuse_pairs):
+        for i in views:
+            same_sources(i, fuse_pairs[i])
+        res = fusion.dtu_filter_views(all_depths, views, confs, table, conf_thres)
+        return {"final": res["final"].unsqueeze(1), "points": res["points"]}
+    fuse.batch = batch
+    return fuse

@@ -388,6 +388,26 @@ int effimvs_dtu_filter_f32(const float* ref_depth, const float* srcs_depth, cons
                            uint8_t* final_mask, uint8_t* geo_mask, float* depth_avg, float* points, uint8_t* masks_out,
                            float* reproj_depth_out, void* stream);
 
+/* The same filter for n reference views of one scene in one launch, reading every depth map in place from one stack.
+ *   depths (n_depths,h,w) fp32: the scene's depth maps (e.g. the all-gathered tensor of the scene runner)
+ *   ref_idx (n) int32: row of view y's reference depth map in `depths`
+ *   src_idx (n,vmax) int32: rows of view y's source depth maps, the first src_count[y] entries used
+ *   src_count (n) int32: view y's source count, in [1, vmax]; vmax in [1,31] (the kernel's histogram limit)
+ *   mats (n, 34 + 50*vmax) fp32: view y's camera pack in the layout of effimvs_dtu_filter_f32 for its src_count[y]
+ *         sources, padded to vmax sources
+ *   conf (n,h,w) fp32 at the depth maps' size
+ *   thresholds, ladder and conf_thres / conf_keep as effimvs_dtu_filter_f32
+ *   -> final_mask (n,h,w) u8, geo_mask (n,h,w) u8 (optional), depth_avg (n,h,w), points (n,3,h,w)
+ * View y's results are bit-identical to effimvs_dtu_filter_f32 on that view alone with the same camera pack.
+ * All index arrays are device arrays and are NOT validated on the device: every entry of ref_idx and of the used part of
+ * src_idx must be in [0, n_depths) and every src_count in [1, vmax] (the caller checks its host lists before uploading).
+ * There is no masks_out / reproj_depth_out here: the per-rung debugging outputs are single-view only. */
+int effimvs_dtu_filter_views_f32(const float* depths, int n_depths, const int* ref_idx, const int* src_idx,
+                                 const int* src_count, int vmax, const float* mats, const float* conf,
+                                 const double* thr_dist_host, const float* thr_diff_host, int n_rungs, int first_rung,
+                                 int full_count, float conf_thres, float conf_keep, int n, int h, int w,
+                                 uint8_t* final_mask, uint8_t* geo_mask, float* depth_avg, float* points, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
