@@ -13,8 +13,6 @@
 // are reused across source views and depth planes.
 // Reductions over the channels of a group and over the views stay in registers; the stage-1
 // kernel reduces softmax statistics over D through shared memory.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "warp_coords.cuh"
 
@@ -381,7 +379,7 @@ extern "C" int effimvs_warp_corr_agg_f32(const float* ref_fea, const float* cons
     int rc = fill_srcs(s, src_fea, n_src);
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    if (nhwc && (C == 8 || C == 16 || C == 32) && ((uintptr_t)ref_fea & 31) == 0 && !getenv("EFFIMVS_WARP_NO_TILE")) {
+    if (nhwc && (C == 8 || C == 16 || C == 32) && ((uintptr_t)ref_fea & 31) == 0) {
         bool aligned = true;
         for (int i = 0; i < n_src; ++i) aligned = aligned && ((uintptr_t)s.p[i] & 31) == 0;   // 256-bit ld.global.nc.v4.b64 in the tile kernels
         if (aligned)
@@ -410,7 +408,7 @@ extern "C" int effimvs_warp_corr_views_f32(const float* ref_fea, const float* co
     int rc = fill_srcs(s, src_fea, n_src);
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    if (fea_layout == EFFIMVS_FEA_NHWC && (C == 8 || C == 16 || C == 32) && ((uintptr_t)ref_fea & 31) == 0 && !getenv("EFFIMVS_WARP_NO_TILE")) {
+    if (fea_layout == EFFIMVS_FEA_NHWC && (C == 8 || C == 16 || C == 32) && ((uintptr_t)ref_fea & 31) == 0) {
         bool aligned = true;
         for (int i = 0; i < n_src; ++i) aligned = aligned && ((uintptr_t)s.p[i] & 31) == 0;   // 256-bit ld.global.nc.v4.b64 in the tile kernels
         if (aligned) return warp_corr_views_tile(ref_fea, s, n_src, proj, hyp, hyp_mode, B, C, H, W, D, sims_out, entropy_out, st);

@@ -1019,34 +1019,15 @@ def test_scene_runner_feature_cache_on_device(hp):
             assert abs(n0 - n1) <= 0.02 * H * W, mode
 
 
-# ---- segment-form warp kernels (csrc/warp_tile.cu: run_round_seg) ---------------------------------------------------
-def _with_env(**kv):
-    import contextlib
-
-    @contextlib.contextmanager
-    def cm():
-        old = {k: os.environ.get(k) for k in kv}
-        os.environ.update({k: str(v) for k, v in kv.items()})
-        try:
-            yield
-        finally:
-            for k, v in old.items():
-                if v is None:
-                    os.environ.pop(k, None)
-                else:
-                    os.environ[k] = v
-    return cm()
-
-
+# ---- channels-last warp kernels (csrc/warp_tile.cu) against the oracle at the cascade's shapes ------------------------
 @pytest.mark.gpu
 @pytest.mark.parametrize("C,D,H,W", [(8, 8, 592, 800), (16, 8, 296, 400), (8, 8, 97, 131), (16, 5, 64, 96), (32, 8, 40, 56), (8, 12, 50, 70)])
 @pytest.mark.parametrize("depth_kind,ratio", [("smooth", 1), ("noise", 1), ("steps", 2), ("smooth", 12), ("near", 1)])
-def test_local_volume_segment_form_vs_oracle(hp, ohp, C, D, H, W, depth_kind, ratio):
-    """a5 through the segment-form kernel (dot products once per source pixel of the epipolar segment's footprint) on
-    channels-last maps: against the oracle on the device, against the plane-by-plane tile kernel and against the gather
-    kernel.  smooth / noise / steps: rendered surface, white-noise depth, depth discontinuities; ratio 12: planes several
-    pixels apart (footprints that do not fit the strip: plane-by-plane path); near: depths so close that most of the
-    segments leave the source images (dead samples, clamped boxes, border cells)."""
+def test_local_volume_channels_last_vs_oracle(hp, ohp, C, D, H, W, depth_kind, ratio):
+    """a5 on channels-last maps (the staged tile kernel) against the oracle on the device, with and without view weights.
+    smooth / noise / steps: rendered surface, white-noise depth, depth discontinuities; ratio 12: planes several pixels
+    apart; near: depths so close that most of the epipolar segments leave the source images (dead samples, clamped boxes,
+    border cells)."""
     from effimvs_b200 import synthetic
     feats, cams, _, wts = synthetic.microbench_inputs(C, D, H, W, views=5, seed=C + D + H, device=DEV)
     gen = torch.Generator().manual_seed(H)
@@ -1065,39 +1046,26 @@ def test_local_volume_segment_form_vs_oracle(hp, ohp, C, D, H, W, depth_kind, ra
     iv = torch.full((1, 1, 1, 1), (1 / 425.0 - 1 / 935.0) / 384 * ratio, device=DEV)
     cl = [f.contiguous(memory_format=torch.channels_last) for f in feats]
     want, want_hyp = ohp.local_volume(cur, feats, cams, iv, wts, D, 1)
-    with _with_env(EFFIMVS_WARP_SEG=1):                       # the segment form is opt-in (the staged tile kernel is the default)
-        got, hyp = hp.local_volume(cur, cl, cams, iv, wts, D, 1)
+    got, hyp = hp.local_volume(cur, cl, cams, iv, wts, D, 1)
     assert torch.equal(hyp, want_hyp)
     assert rel_max(got, want) < 1e-4
-    with _with_env(EFFIMVS_WARP_SEG=0):                       # same coordinates: only fp32 re-association is left
-        tile, _ = hp.local_volume(cur, cl, cams, iv, wts, D, 1)
-    assert rel_max(got, tile) < 2e-6
-    with _with_env(EFFIMVS_WARP_SEG=1, EFFIMVS_WARP_FAST_COORDS=1):   # opt-in: no normalise / un-normalise round trip, one reciprocal
-        fast, _ = hp.local_volume(cur, cl, cams, iv, wts, D, 1)
-    assert rel_max(fast, want) < 1e-3
-    with _with_env(EFFIMVS_WARP_SEG=1):
-        got_nw, _ = hp.local_volume(cur, cl, cams, iv, None, D, 1)
+    got_nw, _ = hp.local_volume(cur, cl, cams, iv, None, D, 1)
     want_nw, _ = ohp.local_volume(cur, feats, cams, iv, None, D, 1)
     assert rel_max(got_nw, want_nw) < 1e-4
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("C,D,H,W,V", [(32, 48, 148, 200, 5), (32, 96, 132, 240, 7), (32, 48, 37, 53, 3), (16, 20, 64, 80, 5)])
-def test_stage1_views_segment_form_vs_oracle(ohp, C, D, H, W, V):
-    """a4 through the segment-form per-view kernel at the DTU and Tanks & Temples stage-1 shapes: per-view similarities and
-    entropies against the oracle on the device and against the plane-by-plane tile kernel."""
+def test_stage1_views_channels_last_vs_oracle(ohp, C, D, H, W, V):
+    """a4 on channels-last maps (the staged per-view tile kernel) at the DTU and Tanks & Temples stage-1 shapes: per-view
+    similarities and entropies against the oracle on the device."""
     from effimvs_b200 import capi, hotpath, ops, synthetic
     feats, cams, hyp, _ = synthetic.microbench_inputs(C, D, H, W, views=V, seed=D, device=DEV)
     feats = [f * 0.4 for f in feats]
     cl = [f.contiguous(memory_format=torch.channels_last) for f in feats]
     planes = hyp[:, :, 0, 0].contiguous()
     proj = hotpath.CudaHotPath().relative_projection(cams)
-    with _with_env(EFFIMVS_WARP_SEG=2):                      # the segment form is opt-in for the per-view kernel
-        sims, ent = ops.warp_corr_views(cl[0], cl[1:], proj, planes, capi.HYP_PLANES, D)
-    with _with_env(EFFIMVS_WARP_SEG=0):
-        sims_t, ent_t = ops.warp_corr_views(cl[0], cl[1:], proj, planes, capi.HYP_PLANES, D)
-    assert rel_max(sims, sims_t) < 2e-6
-    assert rel_max(sims, sims_t) < 1e-4 and float((ent - ent_t).abs().max()) < 1e-3
+    sims, ent = ops.warp_corr_views(cl[0], cl[1:], proj, planes, capi.HYP_PLANES, D)
     for v in range(V - 1):
         want = ohp.view_similarity(feats[0], feats[v + 1], cams[:, 0], cams[:, v + 1], hyp, 1)
         assert rel_max(sims[:, v], want[:, 0]) < 1e-4
@@ -1106,17 +1074,17 @@ def test_stage1_views_segment_form_vs_oracle(ohp, C, D, H, W, V):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("C,D,H,W", [(8, 8, 296, 400), (16, 16, 148, 200), (32, 48, 74, 100)])
-def test_plane_sweep_segment_form_forced(hp, ohp, C, D, H, W):
-    """EFFIMVS_WARP_SEG=2 sends every G = 1 launch (plane sweeps over the whole depth range, explicit per-pixel hypotheses)
-    through the segment form; most footprints do not fit the strip there and take its plane-by-plane path."""
+def test_plane_sweep_channels_last_vs_oracle(hp, ohp, C, D, H, W):
+    """G = 1 plane sweeps over the whole depth range on channels-last maps (the staged tile kernel), with per-pixel
+    hypotheses and with per-batch planes.  At 296 x 400 with 8 planes over the whole range nearly every block's footprint
+    exceeds the staged box, so its samples take the global-gather path."""
     from effimvs_b200 import synthetic
     feats, cams, hyp, wts = synthetic.microbench_inputs(C, D, H, W, views=5, seed=C + D, device=DEV)
     cl = [f.contiguous(memory_format=torch.channels_last) for f in feats]
     sims = [ohp.view_similarity(feats[0], feats[v], cams[:, 0], cams[:, v], hyp, 1) for v in range(1, 5)]
     want = ohp.weighted_aggregate(sims, [wts[:, i:i + 1] for i in range(4)])
-    with _with_env(EFFIMVS_WARP_SEG=2):
-        got = hp.warp_corr_agg(cl, cams, hyp, wts, 1)
-        got_planes = hp.warp_corr_agg(cl, cams, hyp[:, :, :1, :1].contiguous(), wts, 1)
+    got = hp.warp_corr_agg(cl, cams, hyp, wts, 1)
+    got_planes = hp.warp_corr_agg(cl, cams, hyp[:, :, :1, :1].contiguous(), wts, 1)
     assert rel_max(got, want) < 1e-4 and rel_max(got_planes, want) < 1e-4
 
 

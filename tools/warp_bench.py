@@ -64,23 +64,15 @@ def main():
             by = 4.0 * (V * C * H * W + H * W + (V - 1) * H * W + 2 * D * H * W)
         ms_p, out_p = timed(lambda: fn(feats), flush, reps)
         row = {"stage": i + 1, "C": C, "D": D, "H": H, "W": W, "planar_ms": ms_p, "planar_GBs": by / ms_p / 1e6}
-        # channels-last maps: plane-by-plane tile kernel (SEG=0), segment form with fast / upstream-exact coordinates
-        for tag, env in (("tile", {"EFFIMVS_WARP_SEG": "0"}), ("seg", {"EFFIMVS_WARP_SEG": "2"}),
-                         ("seg_fast", {"EFFIMVS_WARP_SEG": "2", "EFFIMVS_WARP_FAST_COORDS": "1"})):
-            os.environ.pop("EFFIMVS_WARP_FAST_COORDS", None)
-            os.environ.update(env)
-            ms_c, out_c = timed(lambda: fn(feats_cl), flush, reps)
-            row.update({tag + "_ms": ms_c, tag + "_GBs": by / ms_c / 1e6,
-                        tag + "_vs_planar_rel_diff": float((out_p - out_c).abs().max() / out_p.abs().max())})
-            if i > 0:      # the same on a smooth surface (what a converged scene looks like)
-                Es, Ks = synthetic.camera_ring(V, W, H)
-                keep = cur
-                cur = synthetic.render_plane_scene(Es[:1], Ks, W, H, noise=0.0)[0].to(dev).reshape(1, 1, H, W)
-                ms_s, _ = timed(lambda: fn(feats_cl), flush, reps)
-                row.update({tag + "_smooth_ms": ms_s, tag + "_smooth_GBs": by / ms_s / 1e6})
-                cur = keep
-        os.environ.pop("EFFIMVS_WARP_FAST_COORDS", None)
-        os.environ.pop("EFFIMVS_WARP_SEG", None)
+        # channels-last maps: the staged tile kernel
+        ms_c, out_c = timed(lambda: fn(feats_cl), flush, reps)
+        row.update({"tile_ms": ms_c, "tile_GBs": by / ms_c / 1e6,
+                    "tile_vs_planar_rel_diff": float((out_p - out_c).abs().max() / out_p.abs().max())})
+        if i > 0:      # the same on a smooth surface (what a converged scene looks like)
+            Es, Ks = synthetic.camera_ring(V, W, H)
+            cur = synthetic.render_plane_scene(Es[:1], Ks, W, H, noise=0.0)[0].to(dev).reshape(1, 1, H, W)
+            ms_s, _ = timed(lambda: fn(feats_cl), flush, reps)
+            row.update({"tile_smooth_ms": ms_s, "tile_smooth_GBs": by / ms_s / 1e6})
         rows.append(row)
         print(json.dumps(row), flush=True)
 
