@@ -92,6 +92,8 @@ SIGNATURES = {
     "effimvs_fusion_invert_cameras_f32": (_i, [_p, _p, _i, _i, _p, _p]),
     "effimvs_fusion_reproject_f32": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p]),
     "effimvs_fusion_filter_f32": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _f, _f, _i, _f, _i, _p, _p, _p, _p, _p]),
+    "effimvs_fusion_filter_views_f32": (_i, [_p, _i, _p, _p, _p, _i, _p, _p, _p, _i, _i, _f, _f, _i, _f, _i, _i, _i, _i,
+                                             _p, _p, _p, _p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

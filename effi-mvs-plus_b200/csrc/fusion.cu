@@ -10,7 +10,8 @@
 //   vote / average / back-projection    upstream test_tank.py:473-515
 //
 // HBM-bound: per reference view it reads (1 + v) depth maps + the confidence map once and
-// writes 1 + 4 + 12 bytes per pixel.
+// writes 1 + 4 + 12 bytes per pixel.  fusion_views_kernel runs the same per-pixel body (fusion_pixel) for all of a
+// scene's reference views in one launch, reading the maps in place from one depth stack through index rows.
 #include "common.cuh"
 
 namespace effimvs {
@@ -227,34 +228,22 @@ __device__ __forceinline__ Reproj reproject(const RefCam& ref, const Cam& src, c
     return r;
 }
 
-template <bool INVERT>
-__global__ void __launch_bounds__(128, 6)
-fusion_kernel(const float* __restrict__ ref_depth, const float* __restrict__ srcs_depth, const float* __restrict__ conf,
-              const float* __restrict__ ref_cam, const float* __restrict__ srcs_cam, const float* __restrict__ inv_cams,
-              int v, int h, int w, int hc, int wc, float dist_base, float rel_diff_base, int thres_view,
-              float prob_threshold, int relative, float inv_half_w, float inv_half_h, float* __restrict__ reproj_xyd, uint8_t* __restrict__ final_mask,
-              float* __restrict__ depth_avg, float* __restrict__ points, uint8_t* __restrict__ masks_out) {
-    __shared__ Cam cams[MAXV + 1];
-    __shared__ float thr_xy[MAXV + 2], thr_d[MAXV + 2];   // the ladder k / dist_base, k / rel_diff_base (fusion.py:172-176) between -inf and +inf
-    const int n = blockIdx.y;
-    const int K = v - thres_view + 1;
-    if (threadIdx.x <= v) {
-        const float* cam = threadIdx.x == 0 ? ref_cam + (size_t)n * 32 : srcs_cam + ((size_t)n * v + threadIdx.x - 1) * 32;
-        const float* inv = inv_cams ? inv_cams + ((size_t)n * (v + 1) + threadIdx.x) * 32 : nullptr;
-        load_cam<INVERT>(cams[threadIdx.x], cam, inv);
-    } else if (threadIdx.x >= 32 && threadIdx.x < 32 + MAXV + 2) {
-        const int j = threadIdx.x - 32, k = j - 1;
-        const float kk = (float)(thres_view + k);
-        thr_xy[j] = j == 0 ? -INFINITY : (k < K ? __fdiv_rn(kk, dist_base) : INFINITY);
-        thr_d[j] = j == 0 ? -INFINITY : (k < K ? __fdiv_rn(kk, rel_diff_base) : INFINITY);
-    }
-    __syncthreads();
+// One reference pixel of the filter (view n of the launch, cameras and ladder already in shared memory).  `ref_of()` is
+// the view's (h,w) reference depth map and `src_of(s)` its source view s's, so the body never knows how the maps are
+// laid out.  conf is (n,hc,wc); the outputs are indexed by n as (n,1,h,w) / (n,3,h,w) / (n,v,3,h,w) / (n,v,K,h,w),
+// and reproj_xyd, final_mask (with depth_avg / points) and masks_out may be null.
+template <class RefOf, class SrcOf>
+__device__ __forceinline__ void fusion_pixel(int n, int pix, const Cam* cams, const float* thr_xy,
+                                             const float* thr_d, RefOf ref_of, SrcOf src_of,
+                                             const float* conf, int v, int K, int h, int w, int hc, int wc,
+                                             float dist_base, float rel_diff_base, int thres_view, float prob_threshold,
+                                             int relative, float inv_half_w, float inv_half_h, float* reproj_xyd,
+                                             uint8_t* final_mask, float* depth_avg,
+                                             float* points, uint8_t* masks_out) {
     const int hw = h * w;
-    const int pix = blockIdx.x * blockDim.x + threadIdx.x;
-    if (pix >= hw) return;
     const int yi = pix / w, xi = pix - yi * w;
     const float cx = (float)xi + 0.5f, cy = (float)yi + 0.5f;
-    const float dref = __ldg(ref_depth + (size_t)n * hw + pix);
+    const float dref = __ldg(ref_of() + pix);
     float ref_world[4];
     img_to_world(cams[0], cx, cy, dref, ref_world);
     RefCam rc;
@@ -270,7 +259,7 @@ fusion_kernel(const float* __restrict__ ref_depth, const float* __restrict__ src
     float sum_d = 0.0f;
     int n_last = 0;
     for (int s = 0; s < v; ++s) {
-        Reproj r = reproject(rc, cams[s + 1], ref_world, srcs_depth + ((size_t)n * v + s) * hw, h, w, inv_half_w, inv_half_h);
+        Reproj r = reproject(rc, cams[s + 1], ref_world, src_of(s), h, w, inv_half_w, inv_half_h);
         if (reproj_xyd) {
             float* o = reproj_xyd + (((size_t)n * v + s) * 3) * hw + pix;
             o[0] = r.x; o[(size_t)hw] = r.y; o[(size_t)2 * hw] = r.d;
@@ -309,6 +298,78 @@ fusion_kernel(const float* __restrict__ ref_depth, const float* __restrict__ src
     points[((size_t)n * 3 + 0) * hw + pix] = pw[0];
     points[((size_t)n * 3 + 1) * hw + pix] = pw[1];
     points[((size_t)n * 3 + 2) * hw + pix] = pw[2];
+}
+
+// the ladder k / dist_base, k / rel_diff_base (fusion.py:172-176) of thres_view <= k < thres_view + K between -inf and +inf,
+// written by threads 32 .. 32 + MAXV + 1 of the block
+__device__ __forceinline__ void fill_ladder(float* __restrict__ thr_xy, float* __restrict__ thr_d, int K, float dist_base,
+                                            float rel_diff_base, int thres_view) {
+    const int j = threadIdx.x - 32, k = j - 1;
+    const float kk = (float)(thres_view + k);
+    thr_xy[j] = j == 0 ? -INFINITY : (k < K ? __fdiv_rn(kk, dist_base) : INFINITY);
+    thr_d[j] = j == 0 ? -INFINITY : (k < K ? __fdiv_rn(kk, rel_diff_base) : INFINITY);
+}
+
+template <bool INVERT>
+__global__ void __launch_bounds__(128, 6)
+fusion_kernel(const float* __restrict__ ref_depth, const float* __restrict__ srcs_depth, const float* __restrict__ conf,
+              const float* __restrict__ ref_cam, const float* __restrict__ srcs_cam, const float* __restrict__ inv_cams,
+              int v, int h, int w, int hc, int wc, float dist_base, float rel_diff_base, int thres_view,
+              float prob_threshold, int relative, float inv_half_w, float inv_half_h, float* __restrict__ reproj_xyd, uint8_t* __restrict__ final_mask,
+              float* __restrict__ depth_avg, float* __restrict__ points, uint8_t* __restrict__ masks_out) {
+    __shared__ Cam cams[MAXV + 1];
+    __shared__ float thr_xy[MAXV + 2], thr_d[MAXV + 2];   // the ladder between -inf and +inf
+    const int n = blockIdx.y;
+    const int K = v - thres_view + 1;
+    if (threadIdx.x <= v) {
+        const float* cam = threadIdx.x == 0 ? ref_cam + (size_t)n * 32 : srcs_cam + ((size_t)n * v + threadIdx.x - 1) * 32;
+        const float* inv = inv_cams ? inv_cams + ((size_t)n * (v + 1) + threadIdx.x) * 32 : nullptr;
+        load_cam<INVERT>(cams[threadIdx.x], cam, inv);
+    } else if (threadIdx.x >= 32 && threadIdx.x < 32 + MAXV + 2) {
+        fill_ladder(thr_xy, thr_d, K, dist_base, rel_diff_base, thres_view);
+    }
+    __syncthreads();
+    const int hw = h * w;
+    const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pix >= hw) return;
+    fusion_pixel(n, pix, cams, thr_xy, thr_d, [=] { return ref_depth + (size_t)n * hw; },
+                 [=](int s) { return srcs_depth + ((size_t)n * v + s) * hw; }, conf, v, K, h, w, hc, wc, dist_base,
+                 rel_diff_base, thres_view, prob_threshold, relative, inv_half_w, inv_half_h, reproj_xyd, final_mask, depth_avg,
+                 points, masks_out);
+}
+
+// Several reference views of one scene in one launch: grid (pixel tiles of 128, n views).  Block y filters reference view
+// y: its reference map is row ref_idx[y] of the one (N,h,w) depth stack, its sources are rows src_idx[y][0 .. src_count[y]),
+// all read in place; the cameras of those rows come from the scene table cams (N,2,4,4) and their inverses from inv_cams
+// (N,2,4,4, as invert_cameras_kernel writes them).  The ladder is the view's own (K = src_count[y] - thres_view + 1).
+// Every view's results are those of fusion_kernel<false> on that view alone with the same cameras and inverses.
+__global__ void __launch_bounds__(128, 6)
+fusion_views_kernel(const float* __restrict__ depths, const int* __restrict__ ref_idx, const int* __restrict__ src_idx,
+                    const int* __restrict__ src_count, int vmax, const float* __restrict__ cam_tab,
+                    const float* __restrict__ inv_tab, const float* __restrict__ conf, int h, int w, int hc, int wc,
+                    float dist_base, float rel_diff_base, int thres_view, float prob_threshold, int relative,
+                    float inv_half_w, float inv_half_h, uint8_t* __restrict__ final_mask, float* __restrict__ depth_avg,
+                    float* __restrict__ points) {
+    __shared__ Cam cams[MAXV + 1];
+    __shared__ float thr_xy[MAXV + 2], thr_d[MAXV + 2];
+    __shared__ int rows[MAXV + 1];                         // stack rows of the reference map, then of the source maps
+    const int n = blockIdx.y;
+    const int v = src_count[n];
+    const int K = v - thres_view + 1;
+    if (threadIdx.x <= v) {
+        const int r = threadIdx.x == 0 ? ref_idx[n] : src_idx[(size_t)n * vmax + threadIdx.x - 1];
+        rows[threadIdx.x] = r;
+        load_cam<false>(cams[threadIdx.x], cam_tab + (size_t)r * 32, inv_tab + (size_t)r * 32);
+    } else if (threadIdx.x >= 32 && threadIdx.x < 32 + MAXV + 2) {
+        fill_ladder(thr_xy, thr_d, K, dist_base, rel_diff_base, thres_view);
+    }
+    __syncthreads();
+    const int hw = h * w;
+    const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pix >= hw) return;
+    fusion_pixel(n, pix, cams, thr_xy, thr_d, [=] { return depths + (size_t)rows[0] * hw; },
+                 [=](int s) { return depths + (size_t)rows[s + 1] * hw; }, conf, v, K, h, w, hc, wc, dist_base, rel_diff_base,
+                 thres_view, prob_threshold, relative, inv_half_w, inv_half_h, nullptr, final_mask, depth_avg, points, nullptr);
 }
 
 // inverse(E), inverse(K) of the 1 + v cameras of every batch item -> inv (n, 1+v, 2, 4, 4), the layout fusion_kernel reads
@@ -414,4 +475,25 @@ extern "C" int effimvs_fusion_masks_f32(const float* ref_depth, const float* rep
     fusion_masks_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(ref_depth, reproj_xyd, v, h, w, dist_base, rel_diff_base, thres_view,
                                                                 relative, masks_out);
     return check_launch("fusion_masks_kernel");
+}
+
+extern "C" int effimvs_fusion_filter_views_f32(const float* depths, int n_depths, const int* ref_idx, const int* src_idx,
+                                               const int* src_count, int vmax, const float* cams, const float* inv_cams,
+                                               const float* conf, int hc, int wc, float dist_base, float rel_diff_base,
+                                               int thres_view, float prob_threshold, int relative, int n, int h, int w,
+                                               uint8_t* final_mask, float* depth_avg, float* points, void* stream) {
+    EFFI_REQUIRE(depths && ref_idx && src_idx && src_count && cams && inv_cams && conf && final_mask && depth_avg && points,
+                 EFFIMVS_EINVAL, "fusion_filter_views: null pointer");
+    EFFI_REQUIRE(n_depths >= 1 && vmax >= 1 && vmax <= MAXV && n >= 1 && n <= 65535 && h > 1 && w > 1 && hc > 0 && wc > 0 &&
+                 (long long)h * w <= 0x7fffffffLL - 127, EFFIMVS_EINVAL,
+                 "fusion_filter_views: bad sizes (N=%d, vmax=%d in [1,%d], n=%d in [1,65535], h=%d, w=%d, hc=%d, wc=%d)",
+                 n_depths, vmax, MAXV, n, h, w, hc, wc);
+    EFFI_REQUIRE(thres_view >= 1 && thres_view <= vmax, EFFIMVS_EINVAL, "fusion_filter_views: thres_view=%d outside [1,%d]", thres_view, vmax);
+    EFFI_REQUIRE(dist_base > 0.0f && rel_diff_base > 0.0f, EFFIMVS_EINVAL, "fusion_filter_views: thresholds must be positive");
+    dim3 block(128), grid(ceil_div(h * w, 128), n);
+    const float ihw = 1.0f / (float)((double)(w - 1) / 2.0), ihh = 1.0f / (float)((double)(h - 1) / 2.0);   // as __fdiv_rn on the device
+    fusion_views_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(depths, ref_idx, src_idx, src_count, vmax, cams, inv_cams, conf, h, w,
+                                                                 hc, wc, dist_base, rel_diff_base, thres_view, prob_threshold, relative,
+                                                                 ihw, ihh, final_mask, depth_avg, points);
+    return check_launch("fusion_views_kernel");
 }

@@ -50,6 +50,128 @@ def filter_view(ref_depth, ref_conf, srcs_depth, ref_cam, srcs_cam, dist_base, r
     return out
 
 
+# ---- the same filter for a whole scene: all of a rank's reference views in one launch -----------------------------
+MAX_SOURCES = 16              # EFFIMVS_MAX_SRC_VIEWS: the camera records a block keeps in shared memory
+
+
+class DynamicSceneCameras:
+    """The dynamic filter's cameras of every view of a scene (see dynamic_scene_cameras).
+
+    cams (N,2,4,4) float32 on the device; inv (N,2,4,4): inverse(E) and inverse(K) (padded to 4x4) of every camera, as
+    effimvs_fusion_invert_cameras_f32 forms them; pairs[i]: the source views of view i (host lists)."""
+
+    def __init__(self, cams: torch.Tensor, inv: torch.Tensor, pairs):
+        self.cams, self.inv = cams, inv
+        self.pairs = [[int(j) for j in p] for p in pairs]
+        self.n_views = len(self.pairs)
+        self.vmax = max(len(p) for p in self.pairs)
+        self._rows = {}
+
+    def check(self, views, thres_view: int):
+        """ValueError naming the first of `views` that is outside the scene or has fewer than thres_view sources"""
+        for i in views:
+            if not 0 <= i < self.n_views:
+                raise ValueError("view {} is outside the scene's {} views".format(i, self.n_views))
+            if len(self.pairs[i]) < thres_view:
+                raise ValueError("view {} has {} source views, fewer than thres_view = {}".format(i, len(self.pairs[i]), thres_view))
+
+    def rows(self, views, device, stack_rows=None, n_stack=None):
+        """the device arrays of effimvs_fusion_filter_views_f32 for reference views `views` (in that order):
+        (ref_idx (n,), src_idx (n,vmax), src_count (n,) int32, cams (N,2,4,4), inv (N,2,4,4)).  Indices are scene view
+        numbers, or stack_rows[view] where the depth stack (n_stack maps) holds the scene's maps in another order; then
+        cams / inv are gathered into the stack's order.  Built and uploaded in one host -> device copy the first time a
+        list is asked for, then cached: a host -> device copy synchronises the host with the stream and cannot be
+        captured in a CUDA graph, so the first call for a list comes before a capture."""
+        views = [int(i) for i in views]
+        key = (tuple(views), str(device), None if stack_rows is None else (tuple(sorted(stack_rows.items())), n_stack))
+        if key not in self._rows:
+            self.check(views, 0)
+            row = (lambda j: j) if stack_rows is None else (lambda j: int(stack_rows[j]))   # noqa: E731
+            n, vmax = len(views), self.vmax
+            host = [row(i) for i in views]
+            for i in views:
+                host += [row(j) for j in self.pairs[i]] + [0] * (vmax - len(self.pairs[i]))
+            host += [len(self.pairs[i]) for i in views]
+            if stack_rows is not None:          # the scene view of every stack row this launch reads (others: view 0)
+                perm = [0] * n_stack
+                for i in views:
+                    for j in [i] + self.pairs[i]:
+                        perm[row(j)] = j
+                host += perm
+            dev = torch.as_tensor(host, dtype=torch.int32).to(device)
+            a, b, c = n, n + n * vmax, 2 * n + n * vmax
+            cams, inv = self.cams, self.inv
+            if stack_rows is not None:
+                cams, inv = cams.index_select(0, dev[c:]), inv.index_select(0, dev[c:])
+            self._rows[key] = (dev[:a], dev[a:b].view(n, vmax), dev[b:c], cams, inv)
+        return self._rows[key]
+
+
+def dynamic_scene_cameras(cams_stage4: torch.Tensor, fuse_pairs) -> DynamicSceneCameras:
+    """Cameras of every view of a scene for the batched dynamic filter.  cams_stage4 (N,2,4,4) on the device (E = [:, 0],
+    K = [:, 1, :3, :3], the full-resolution cameras filter_view takes); fuse_pairs[i]: the 1 .. 16 source views of view i.
+    The inverse table is built in one launch of effimvs_fusion_invert_cameras_f32, the kernel filter_view(...,
+    torch_inverse=False) inverts every view's cameras with, so the batched results are bit-identical to it."""
+    if cams_stage4.dim() != 4 or tuple(cams_stage4.shape[1:]) != (2, 4, 4):
+        raise ValueError("cams_stage4 must be (N,2,4,4), got {}".format(tuple(cams_stage4.shape)))
+    N = cams_stage4.shape[0]
+    if len(fuse_pairs) != N:
+        raise ValueError("{} source lists for {} views".format(len(fuse_pairs), N))
+    pairs = [[int(j) for j in p] for p in fuse_pairs]
+    for i, p in enumerate(pairs):
+        if not 1 <= len(p) <= MAX_SOURCES:
+            raise ValueError("view {} has {} source views; the dynamic filter takes 1 to {}".format(i, len(p), MAX_SOURCES))
+        if any(not 0 <= j < N for j in p):
+            raise ValueError("view {}: source views {} are outside the scene's {} views".format(i, p, N))
+    cams = cams_stage4.detach().float().contiguous()
+    inv = ops.fusion_invert_cameras(cams, cams.unsqueeze(1))[:, 0].contiguous()     # (N, 2, 2,4,4): column 0 is camera i's
+    return DynamicSceneCameras(cams, inv, pairs)
+
+
+def filter_views(depth_stack, views, confs, table: DynamicSceneCameras, dist_base, rel_diff_base, thres_view, prob_threshold,
+                 relative: bool = False, stack_rows=None):
+    """``dynamic_filter_depth`` (test_tank.py:470-515) for the reference views `views` in ONE launch.
+
+    depth_stack (N,h,w) CUDA fp32 holds the depth map of every view of the scene (the scene runner's all-gathered maps);
+    each view's reference and source maps are read from it in place.  stack_rows: {view: row of depth_stack} when the
+    stack is not in scene order (default: view i is row i, and N is the scene's view count).  confs (n,hc,wc) CUDA fp32,
+    nearest-resized to (h,w) in the kernel as filter_view does; table from dynamic_scene_cameras.  Makes no host
+    synchronisation once the table's rows for `views` are on the device (table.rows), so it can be captured in a CUDA
+    graph.  -> dict(final (n,1,h,w) bool, depth_avg (n,1,h,w), points (n,3,h,w)); view views[b]'s results are
+    bit-identical to filter_view(..., torch_inverse=False) on that view alone."""
+    views = [int(i) for i in views]
+    if not views:
+        raise ValueError("no reference view to filter")
+    if len(views) > 65535:
+        raise ValueError("{} reference views in one launch; at most 65535".format(len(views)))
+    thres_view = int(thres_view)
+    if thres_view < 1:
+        raise ValueError("thres_view must be at least 1, got {}".format(thres_view))
+    if not (dist_base > 0 and rel_diff_base > 0):
+        raise ValueError("dist_base and rel_diff_base must be positive, got {} and {}".format(dist_base, rel_diff_base))
+    table.check(views, thres_view)
+    if depth_stack.dim() != 3:
+        raise ValueError("depth_stack must be (N,h,w), got {}".format(tuple(depth_stack.shape)))
+    N, h, w = depth_stack.shape
+    if stack_rows is None and N != table.n_views:
+        raise ValueError("the depth stack holds {} maps, the camera table {} views".format(N, table.n_views))
+    if stack_rows is not None:
+        for i in views:
+            need = [i] + table.pairs[i]
+            if any(j not in stack_rows or not 0 <= stack_rows[j] < N for j in need):
+                raise ValueError("view {}: views {} are not all rows of the {}-map depth stack".format(i, need, N))
+        need = sorted({j for i in views for j in [i] + table.pairs[i]})
+        if len({stack_rows[j] for j in need}) != len(need):
+            raise ValueError("views {} do not have a depth-stack row each".format(need))
+    n = len(views)
+    if confs.dim() != 3 or confs.shape[0] != n:
+        raise ValueError("confs must be (n,hc,wc) for n = {} views, got {}".format(n, tuple(confs.shape)))
+    ref, src, count, cams, inv = table.rows(views, depth_stack.device, stack_rows, N)
+    final, avg, pts = ops.fusion_filter_views(depth_stack, ref, src, count, cams, inv, confs, float(dist_base), float(rel_diff_base),
+                                              thres_view, float(prob_threshold), bool(relative))
+    return {"final": final.bool(), "depth_avg": avg, "points": pts}
+
+
 # ---- SURVEY section 8(f) row 2: the DTU pipeline's filter (test_dtu_dypcd.py:164-350) ---------------------------
 DTU_FIRST_RUNG, DTU_END_RUNG = 1, 11          # s, e (test_dtu_dypcd.py:33-34)
 DTU_DIST_BASE, DTU_DIFF_BASE = 1 / 2, 0.25    # :36-37

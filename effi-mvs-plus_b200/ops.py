@@ -1111,3 +1111,38 @@ def _(depths, ref_idx, src_idx, src_count, mats, conf, thr_dist, thr_diff, first
     u8 = torch.uint8
     return (depths.new_empty(n, h, w, dtype=u8), depths.new_empty(n, h, w, dtype=u8), depths.new_empty(n, h, w),
             depths.new_empty(n, 3, h, w))
+
+
+@torch.library.custom_op("effimvs::fusion_filter_views", mutates_args=())
+@_on_tensor_device
+def fusion_filter_views(depths: Tensor, ref_idx: Tensor, src_idx: Tensor, src_count: Tensor, cams: Tensor, inv_cams: Tensor,
+                        conf: Tensor, dist_base: float, rel_diff_base: float, thres_view: int, prob_threshold: float,
+                        relative: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """n reference views of one scene in one launch of the dynamic filter.  depths (N,h,w); ref_idx (n), src_idx (n,vmax),
+    src_count (n) int32 rows of `depths` (NOT checked on the device: the caller validates its host lists); cams, inv_cams
+    (N,2,4,4): the camera of every row of `depths` and its inverses; conf (n,hc,wc).
+    -> final (n,1,h,w) u8, depth_avg (n,1,h,w), points (n,3,h,w)."""
+    name = "fusion_filter_views"
+    depths, cams, inv_cams, conf = _dev(depths, name), _dev(cams, name), _dev(inv_cams, name), _dev(conf, name)
+    ref_idx, src_idx, src_count = _dev_i32(ref_idx, name), _dev_i32(src_idx, name), _dev_i32(src_count, name)
+    N, h, w = depths.shape
+    n, vmax = src_idx.shape
+    hc, wc = conf.shape[-2:]
+    dev = depths.device
+    final = torch.empty(n, 1, h, w, device=dev, dtype=torch.uint8)
+    avg = torch.empty(n, 1, h, w, device=dev, dtype=torch.float32)
+    pts = torch.empty(n, 3, h, w, device=dev, dtype=torch.float32)
+    _count(1)
+    capi.check(_lib.effimvs_fusion_filter_views_f32(depths.data_ptr(), N, ref_idx.data_ptr(), src_idx.data_ptr(),
+                                                    src_count.data_ptr(), vmax, cams.data_ptr(), inv_cams.data_ptr(),
+                                                    conf.data_ptr(), hc, wc, dist_base, rel_diff_base, thres_view,
+                                                    prob_threshold, int(relative), n, h, w, final.data_ptr(), avg.data_ptr(),
+                                                    pts.data_ptr(), _stream()))
+    return final, avg, pts
+
+
+@fusion_filter_views.register_fake
+def _(depths, ref_idx, src_idx, src_count, cams, inv_cams, conf, dist_base, rel_diff_base, thres_view, prob_threshold, relative):
+    _, h, w = depths.shape
+    n = src_idx.shape[0]
+    return depths.new_empty(n, 1, h, w, dtype=torch.uint8), depths.new_empty(n, 1, h, w), depths.new_empty(n, 3, h, w)

@@ -294,7 +294,9 @@ def cuda_scene_callables(model, imgs: torch.Tensor, cams: Dict[str, torch.Tensor
     that lists it as a source (section 8(f) row 1; eval-mode results are those of re-encoding it).
     graphed_src_views > 0: run encode / cascade as CUDA graphs captured for that many source views (implies the
     feature cache); then infer.batch([(ref_view, src_views), ...]) runs up to views_per_replay views per replay of the
-    cascade, and run_scene groups the views accordingly.  views_per_replay > 1 needs the graphs."""
+    cascade, and run_scene groups the views accordingly.  views_per_replay > 1 needs the graphs.
+    fuse(i, ...) filters one view (fusion.filter_view); fuse.batch(views, all_depths, confs, fuse_pairs) filters all of a
+    rank's views in one launch (fusion.filter_views), and run_scene calls it instead of fuse per view."""
     from . import fusion
     if views_per_replay != 1 and graphed_src_views <= 0:
         raise ValueError("views_per_replay = {} needs graphed_src_views > 0 (views are batched inside the CUDA graph)".format(views_per_replay))
@@ -339,6 +341,19 @@ def cuda_scene_callables(model, imgs: torch.Tensor, cams: Dict[str, torch.Tensor
             sel_cache[key] = torch.as_tensor(list(srcs), device=full.device)
         return fusion.filter_view(ref_depth, conf, src_depths, full[i].unsqueeze(0), full.index_select(0, sel_cache[key]).unsqueeze(0),
                                   dist_base, rel_diff_base, thres_view, prob_threshold, torch_inverse=False)
+
+    tables: Dict[tuple, "fusion.DynamicSceneCameras"] = {}
+
+    def fuse_batch(views, all_depths, confs, fuse_pairs):
+        """all of a rank's views in one launch of the same filter (run_scene's batched fuse protocol): the scene's camera
+        table is built once per distinct fuse_pairs, the depth maps are read in place from the all-gathered tensor, and
+        every view's points are bit-identical to those of the per-view fuse"""
+        key = tuple(tuple(int(j) for j in p) for p in fuse_pairs)
+        if key not in tables:
+            tables[key] = fusion.dynamic_scene_cameras(cams["stage4"], key)
+        res = fusion.filter_views(all_depths, views, confs, tables[key], dist_base, rel_diff_base, thres_view, prob_threshold)
+        return {"final": res["final"], "points": res["points"]}
+    fuse.batch = fuse_batch
     return infer, fuse
 
 

@@ -235,6 +235,29 @@ int effimvs_fusion_filter_f32(const float* ref_depth, const float* srcs_depth, c
                               int relative, uint8_t* final_mask, float* depth_avg, float* points,
                               uint8_t* masks_out, void* stream);
 
+/* The same filter for n reference views of one scene in one launch, reading every depth map in place from one stack.
+ *   depths (n_depths,h,w) fp32: the scene's depth maps (e.g. the all-gathered tensor of the scene runner)
+ *   ref_idx (n) int32: row of view y's reference depth map in `depths`
+ *   src_idx (n,vmax) int32: rows of view y's source depth maps, the first src_count[y] entries used
+ *   src_count (n) int32: view y's source count, in [thres_view, vmax]; vmax in [1,16] (EFFIMVS_MAX_SRC_VIEWS)
+ *   cams (n_depths,2,4,4) fp32: the camera of every row of `depths`, as ref_cam / srcs_cam of effimvs_fusion_filter_f32
+ *   inv_cams (n_depths,2,4,4) fp32: their inverses in the layout of effimvs_fusion_invert_cameras_f32 (for instance its
+ *         output for ref_cam = cams, v = 1, column 0)
+ *   conf (n,hc,wc) fp32, nearest-resized to (h,w); thresholds, thres_view, prob_threshold and relative as
+ *         effimvs_fusion_filter_f32 (the ladder of view y has K = src_count[y] - thres_view + 1 rungs)
+ *   -> final_mask (n,h,w) u8, depth_avg (n,h,w), points (n,3,h,w)
+ * View y's results are bit-identical to effimvs_fusion_filter_f32 on that view alone with the same cameras and inverses.
+ * The host rejects null pointers, vmax outside [1,16], n outside [1,65535], non-positive sizes, non-positive bases and
+ * thres_view outside [1,vmax].  All index arrays are device arrays and are NOT validated on the device: every entry of
+ * ref_idx and of the used part of src_idx must be in [0, n_depths), and thres_view <= src_count[y] <= vmax for every y
+ * (the caller checks its host lists before uploading).  There is no masks_out / reproj_xyd here: the per-rung debugging
+ * outputs are single-view only. */
+int effimvs_fusion_filter_views_f32(const float* depths, int n_depths, const int* ref_idx, const int* src_idx,
+                                    const int* src_count, int vmax, const float* cams, const float* inv_cams,
+                                    const float* conf, int hc, int wc, float dist_base, float rel_diff_base,
+                                    int thres_view, float prob_threshold, int relative, int n, int h, int w,
+                                    uint8_t* final_mask, float* depth_avg, float* points, void* stream);
+
 /* ---- SURVEY section 8(f) row 3: per-pixel glue of the ConvGRU update block and convex upsampling --------
  * The 2-D convolutions stay cuDNN on the upstream side; these entry points replace the elementwise
  * chains between them.  Multi-channel maps are channels-last (B,H,W,C). */
