@@ -94,6 +94,9 @@ SIGNATURES = {
     "effimvs_fusion_filter_f32": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _f, _f, _i, _f, _i, _p, _p, _p, _p, _p]),
     "effimvs_fusion_filter_views_f32": (_i, [_p, _i, _p, _p, _p, _i, _p, _p, _p, _i, _i, _f, _f, _i, _f, _i, _i, _i, _i,
                                              _p, _p, _p, _p]),
+    "effimvs_point_offsets_workspace_bytes": (_sz, [_i, _i, _i]),
+    "effimvs_point_offsets": (_i, [_p, _i, _i, _i, _p, _sz, _p, _p]),
+    "effimvs_gather_points_f32": (_i, [_p, _p, _p, _i, _p, _i, _i, _i, _p, _sz, _p, _p, _p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

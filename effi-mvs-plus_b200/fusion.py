@@ -330,3 +330,54 @@ def dtu_filter_views(depth_stack, views, confs, table: DtuSceneCameras, conf_thr
     final, geo, avg, pts = ops.dtu_filter_views(depth_stack, ref, src, count, mats, confs, thr_dist, thr_diff, first_rung,
                                                 end_rung, float(conf_thres), 0.75)
     return {"final": final.bool(), "geo": geo.bool(), "depth_avg": avg, "points": pts}
+
+
+# ---- the scene's coloured point cloud (test_tank.py:517-570, test_dtu_dypcd.py:339-350) ---------------------------
+_IMAGE_ROWS = {}          # (views, device) -> (n,) int32 device copy of the image row of every view
+
+
+def require_cuda(*tensors):
+    """the library's CUDA-only error for any CPU tensor among `tensors` (None entries are skipped)"""
+    if any(t is not None and not t.is_cuda for t in tensors):
+        raise RuntimeError("effimvs::compact_points got a CPU tensor; the hot path is CUDA-only (no fallback)")
+
+
+def compact_points(final, points, views, images=None):
+    """Upstream's vertex and colour collection for n reference views in three launches: the kept points of every view,
+    in the order of `views` and in raster order within a view -- bit for bit ``points[b][:, final[b]].t()`` per view --
+    and their colours from the reference images.
+
+    final (n,h,w) or (n,1,h,w) bool and points (n,3,h,w) fp32 CUDA, as filter_views / dtu_filter_views return them;
+    views: the scene view number of each of the n rows (the row of `images` its colours come from); images (N,3,h,w) fp32
+    CUDA, e.g. run_scene's, or None for points only.  A colour byte is trunc(clamp(image * 255, 0, 255)) (NaN: 0), which
+    on [0,1] is NumPy's (image * 255).astype(np.uint8) and gives back the byte of a u8 / 255 image.
+    -> (points (total,3) fp32, colors (total,3) uint8 or None, offsets: host list of n+1 ints, view b's points being rows
+    offsets[b] .. offsets[b+1] - 1).  The one host synchronisation is the read of the offsets, which sizes the outputs.
+    The device copy of the image rows is made once per distinct `views` and cached."""
+    views = [int(i) for i in views]
+    if not views:
+        raise ValueError("no view to take points from")
+    if final.dim() == 4 and final.shape[1] == 1:
+        final = final.reshape(final.shape[0], *final.shape[2:])
+    if final.dim() != 3 or points.dim() != 4 or tuple(points.shape) != (final.shape[0], 3, *final.shape[1:]):
+        raise ValueError("final (n,h,w) and points (n,3,h,w) of the same n, h, w, got {} and {}".format(tuple(final.shape),
+                                                                                                         tuple(points.shape)))
+    n, h, w = final.shape
+    if len(views) != n:
+        raise ValueError("{} views for {} masks".format(len(views), n))
+    if images is not None:
+        if images.dim() != 4 or images.shape[1] != 3 or tuple(images.shape[-2:]) != (h, w):
+            raise ValueError("images must be (N,3,{},{}) like the depth maps, got {}".format(h, w, tuple(images.shape)))
+        if any(not 0 <= i < images.shape[0] for i in views):
+            raise ValueError("views {} are not all rows of the {} images".format(views, images.shape[0]))
+    require_cuda(final, points, images)
+    rows = None
+    if images is not None:
+        key = (tuple(views), str(images.device))
+        if key not in _IMAGE_ROWS:
+            _IMAGE_ROWS[key] = torch.as_tensor(views, dtype=torch.int32).to(images.device)
+        rows = _IMAGE_ROWS[key]
+    view_offsets, ws = ops.point_offsets(final)
+    offsets = view_offsets.cpu().tolist()
+    pts, colors = ops.gather_points(final, points, images, rows, ws, offsets[-1])
+    return pts, (colors if images is not None else None), offsets

@@ -1146,3 +1146,76 @@ def _(depths, ref_idx, src_idx, src_count, cams, inv_cams, conf, dist_base, rel_
     _, h, w = depths.shape
     n = src_idx.shape[0]
     return depths.new_empty(n, 1, h, w, dtype=torch.uint8), depths.new_empty(n, 1, h, w), depths.new_empty(n, 3, h, w)
+
+
+# -------------------------------------------------------------------------------------------
+# the scene's coloured point cloud (csrc/points.cu): stream compaction of the filters' dense outputs
+def _mask_u8(t: Tensor, name: str) -> Tensor:
+    if not t.is_cuda:
+        raise RuntimeError("effimvs::{} got a CPU tensor; the hot path is CUDA-only (no fallback)".format(name))
+    t = t.contiguous()
+    return t.view(torch.uint8) if t.dtype == torch.bool else t.to(torch.uint8)
+
+
+def point_offsets_workspace_bytes(n: int, h: int, w: int) -> int:
+    return int(_lib.effimvs_point_offsets_workspace_bytes(n, h, w))
+
+
+@torch.library.custom_op("effimvs::point_offsets", mutates_args=())
+@_on_tensor_device
+def point_offsets(final: Tensor) -> Tuple[Tensor, Tensor]:
+    """final (n,h,w) bool / uint8 (nonzero = kept) -> view_offsets (n+1) int64 (view y's points are rows
+    view_offsets[y] .. view_offsets[y+1] - 1, view_offsets[n] the total) and offsets_ws, the tile workspace
+    gather_points reads.  Two launches, no host synchronisation."""
+    final = _mask_u8(final, "point_offsets")
+    n, h, w = final.shape
+    ws = torch.empty(point_offsets_workspace_bytes(n, h, w), device=final.device, dtype=torch.uint8)
+    offsets = torch.empty(n + 1, device=final.device, dtype=torch.int64)
+    _count(2)
+    capi.check(_lib.effimvs_point_offsets(final.data_ptr(), n, h, w, ws.data_ptr(), ws.numel(), offsets.data_ptr(), _stream()))
+    return offsets, ws
+
+
+@point_offsets.register_fake
+def _(final):
+    n, h, w = final.shape
+    return final.new_empty(n + 1, dtype=torch.int64), final.new_empty(point_offsets_workspace_bytes(n, h, w), dtype=torch.uint8)
+
+
+@torch.library.custom_op("effimvs::gather_points", mutates_args=())
+@_on_tensor_device
+def gather_points(final: Tensor, points: Tensor, images: Optional[Tensor], image_rows: Optional[Tensor], offsets_ws: Tensor,
+                  total: int) -> Tuple[Tensor, Tensor]:
+    """The kept points of final (n,h,w) from points (n,3,h,w), in view order and raster order within a view, and their
+    colours from images (n_images,3,h,w) fp32 rows image_rows (n) int32 (NOT checked on the device: the caller validates
+    its host list).  offsets_ws: point_offsets' workspace for this mask; total: its view_offsets[n].
+    -> points (total,3) fp32, colors (total,3) uint8 ((0,3) without images).  One launch (none when total is 0)."""
+    name = "gather_points"
+    final, points = _mask_u8(final, name), _dev(points, name)
+    if not offsets_ws.is_cuda:
+        raise RuntimeError("effimvs::{} got a CPU tensor; the hot path is CUDA-only (no fallback)".format(name))
+    n, h, w = final.shape
+    if tuple(points.shape) != (n, 3, h, w) or (images is not None and (images.dim() != 4 or tuple(images.shape[1:]) != (3, h, w)
+                                                                       or image_rows is None or image_rows.numel() != n)):
+        raise ValueError("effimvs::gather_points: mask (n,h,w), points (n,3,h,w), images (N,3,h,w) and n image rows, got {}, {}, {}, {}"
+                         .format(tuple(final.shape), tuple(points.shape), None if images is None else tuple(images.shape),
+                                 None if image_rows is None else tuple(image_rows.shape)))
+    dev = final.device
+    out = torch.empty(total, 3, device=dev, dtype=torch.float32)
+    colors = torch.empty(total if images is not None else 0, 3, device=dev, dtype=torch.uint8)
+    n_images = 0
+    if images is not None:
+        images, image_rows = _dev(images, name), _dev_i32(image_rows, name)
+        n_images = images.shape[0]
+    if total == 0:
+        return out, colors
+    _count(1)
+    capi.check(_lib.effimvs_gather_points_f32(final.data_ptr(), points.data_ptr(), _opt(images), n_images, _opt(image_rows), n, h, w,
+                                              offsets_ws.data_ptr(), offsets_ws.numel(), out.data_ptr(),
+                                              colors.data_ptr() if images is not None else None, _stream()))
+    return out, colors
+
+
+@gather_points.register_fake
+def _(final, points, images, image_rows, offsets_ws, total):
+    return points.new_empty(total, 3), points.new_empty(total if images is not None else 0, 3, dtype=torch.uint8)

@@ -92,7 +92,7 @@ def agree_on_size(local_hw, n_views: int, world: int, device):
 @torch.no_grad()
 def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Sequence[int]], rank: int = 0, world: int = 1,
               device="cuda", fuse_pairs: Sequence[Sequence[int]] = None, timings: dict = None, sharding: str = "round_robin",
-              views_per_batch: int = None):
+              views_per_batch: int = None, images: torch.Tensor = None):
     """infer(ref_view, src_views) -> (depth (h,w), conf (hc,wc)) on `device`;
     fuse(ref_view, ref_depth (1,1,h,w), conf (1,hc,wc), src_views, src_depths (1,v,1,h,w)) -> dict with
     'final' (1,1,h,w) bool and 'points' (1,3,h,w).
@@ -103,8 +103,18 @@ def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Seq
     When fuse has `batch`, it is called once for all of the rank's views instead of fuse per view:
     fuse.batch(views in order, all depth maps (n_views,h,w), confs (n,hc,wc), fuse_pairs) -> dict with 'final'
     (n,1,h,w) bool and 'points' (n,3,h,w).
-    Returns {ref_view: (points (k,3), depth (h,w))} for the views this rank owns."""
+    Returns {ref_view: (points (k,3), depth (h,w))} for the views this rank owns.
+    images (n_views,3,h,w) fp32 CUDA, the reference images at the depth maps' size (cuda_scene_callables' `imgs`): each
+    entry is then (points (k,3), depth (h,w), colors (k,3) uint8), the points compacted on the device by
+    fusion.compact_points -- one pass for all of the rank's views with fuse.batch (the entries are slices of one buffer),
+    one per view otherwise -- bit-identical to those without images.  A rank's cloud in upstream's vertex order:
+    data_io.write_ply(path, torch.cat(points).cpu(), torch.cat(colors).cpu()) over its views in order."""
     fuse_pairs = pairs if fuse_pairs is None else fuse_pairs
+    if images is not None:
+        from . import fusion
+        if images.dim() != 4 or tuple(images.shape[:2]) != (n_views, 3):
+            raise ValueError("images must be ({},3,h,w), got {}".format(n_views, tuple(images.shape)))
+        fusion.require_cuda(images)
     mine = shard_views(n_views, rank, world, sharding)
     batch = getattr(infer, "batch", None)
     k = views_per_batch if views_per_batch is not None else getattr(infer, "views_per_batch", 1)
@@ -125,6 +135,8 @@ def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Seq
                 depths[i], confs[i] = d, c
     # a rank without a view (n_views < world) still enters the collective below with a zero block
     h, w = agree_on_size(tuple(next(iter(depths.values())).shape[-2:]) if depths else None, n_views, world, device)
+    if images is not None and tuple(images.shape[-2:]) != (h, w):
+        raise ValueError("images are {}x{}, the depth maps {}x{}".format(images.shape[-1], images.shape[-2], w, h))
     ev = None
     if timed:
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
@@ -137,9 +149,14 @@ def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Seq
     if fuse_batch is not None:
         if mine:
             res = fuse_batch(mine, all_depths, torch.stack([confs[i] for i in mine]), fuse_pairs)
-            for b, i in enumerate(mine):
-                m = res["final"][b, 0]
-                out[i] = (res["points"][b][:, m].t().contiguous(), depths[i])
+            if images is None:
+                for b, i in enumerate(mine):
+                    m = res["final"][b, 0]
+                    out[i] = (res["points"][b][:, m].t().contiguous(), depths[i])
+            else:
+                pts, colors, at = fusion.compact_points(res["final"], res["points"], mine, images)
+                for b, i in enumerate(mine):
+                    out[i] = (pts[at[b]:at[b + 1]], depths[i], colors[at[b]:at[b + 1]])
     else:
         flat = [j for i in mine for j in fuse_pairs[i]]
         flat_dev = torch.as_tensor(flat, device=all_depths.device, dtype=torch.long) if flat else None      # ONE host -> device copy
@@ -149,8 +166,12 @@ def run_scene(infer: Callable, fuse: Callable, n_views: int, pairs: Sequence[Seq
             sel = flat_dev[at:at + len(src)]
             at += len(src)
             res = fuse(i, depths[i].reshape(1, 1, h, w), confs[i].unsqueeze(0), src, all_depths.index_select(0, sel).reshape(1, len(src), 1, h, w))
-            m = res["final"][0, 0]
-            out[i] = (res["points"][0][:, m].t().contiguous(), depths[i])
+            if images is None:
+                m = res["final"][0, 0]
+                out[i] = (res["points"][0][:, m].t().contiguous(), depths[i])
+            else:
+                pts, colors, _ = fusion.compact_points(res["final"], res["points"], [i], images)
+                out[i] = (pts, depths[i], colors)
     if ev:
         ev[2].record()
         torch.cuda.synchronize()

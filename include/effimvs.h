@@ -431,6 +431,36 @@ int effimvs_dtu_filter_views_f32(const float* depths, int n_depths, const int* r
                                  int full_count, float conf_thres, float conf_keep, int n, int h, int w,
                                  uint8_t* final_mask, uint8_t* geo_mask, float* depth_avg, float* points, void* stream);
 
+/* ---- the scene's coloured point cloud (upstream's vertex / colour collection, test_tank.py:517-570,
+ * test_dtu_dypcd.py:339-350): stream compaction of the filters' dense outputs for n reference views ----------------
+ * Views come in the order given; within a view, points come in raster order (row-major over (h,w)).  Offsets come from a
+ * scan, never from atomics: two runs give the same bits.  Points are copied, never computed.  Two calls, three launches:
+ *
+ * Bytes of the tile workspace both calls share (8 per 4096-pixel tile of every view); 0 for bad sizes. */
+size_t effimvs_point_offsets_workspace_bytes(int n, int h, int w);
+
+/*   final_mask (n,h,w) uint8: the filters' final masks (nonzero = kept), as effimvs_fusion_filter_views_f32 and
+ *         effimvs_dtu_filter_views_f32 write them
+ *   workspace: effimvs_point_offsets_workspace_bytes(n, h, w) bytes of device memory, 16-byte aligned; receives the
+ *         offset of every tile's first point, which effimvs_gather_points_f32 reads
+ *   -> view_offsets (n+1) int64 device array: view y's points are rows view_offsets[y] .. view_offsets[y+1] - 1 of the
+ *         output, view_offsets[n] is the total.  Two launches (count, scan). */
+int effimvs_point_offsets(const uint8_t* final_mask, int n, int h, int w, void* workspace, size_t workspace_bytes,
+                          int64_t* view_offsets, void* stream);
+
+/*   final_mask (n,h,w) uint8 and workspace as effimvs_point_offsets left them
+ *   points (n,3,h,w) fp32: the filters' world points
+ *   images (n_images,3,h,w) fp32 reference images, or NULL for points only (then image_rows and colors_out are ignored)
+ *   image_rows (n) int32 device array: the row of `images` holding view y's image (e.g. its scene view number).  NOT
+ *         validated on the device: every entry must be in [0, n_images) (the caller checks its host list before uploading)
+ *   -> points_out (total,3) fp32, colors_out (total,3) uint8, both 16-byte aligned, total = view_offsets[n].
+ *      Colour channel c is image channel c: trunc(clamp(image * 255, 0, 255)) with an IEEE fp32 multiply, NaN giving 0.
+ *      On [0,1] that is NumPy's (image * 255).astype(np.uint8), and it returns the byte of every u8 / 255 image; outside
+ *      [0,1] (where NumPy's cast is undefined) the clamp is this library's definition.  One launch. */
+int effimvs_gather_points_f32(const uint8_t* final_mask, const float* points, const float* images, int n_images,
+                              const int* image_rows, int n, int h, int w, const void* workspace, size_t workspace_bytes,
+                              float* points_out, uint8_t* colors_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
